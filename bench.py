@@ -197,7 +197,8 @@ def reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 10); c3 / c4 / c5: timed passes over the list (default 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="c2", choices=list(WORKLOADS) + list(LIST_WORKLOADS))
     ap.add_argument("--list-videos", type=int, default=0, help="c3 / c4: number of videos in the list (default 16 / 512)")
@@ -220,7 +221,15 @@ def main():
                     help="host staging pool of the e2e leg: huge-page mapping + cudaHostRegister, or torch pin_memory")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-k1", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (batch workloads: rank 0's batch)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 1 if args.workload in LIST_WORKLOADS and args.impl == "ours" else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.workload in LIST_WORKLOADS:
@@ -285,6 +294,8 @@ def main():
     e1.record()
     barrier()
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch)
     if args.graph:                       # per-stage times of the same work, outside the timed region
         for _ in range(3):
             batch.run(params, timers=timers)
@@ -385,6 +396,80 @@ def main():
         dist.destroy_process_group()
 
 
+DUMP_BUDGET = 60_000_000          # bytes of all --dump-outputs files together
+
+
+def write_arrays(out_dir, src, budget=DUMP_BUDGET, seed=0):
+    """One out_dir/<name>.npy per entry of `src` (name -> (rows, bytes per row, get(row indices or None) -> array)). The
+    arrays share `budget` bytes, smallest first; one that does not fit its share is replaced by rows drawn with a fixed
+    seed, whose row numbers go to <name>_rows.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = budget
+    for i, name in enumerate(sorted(src, key=lambda k: src[k][0] * src[k][1])):
+        nrows, row_bytes, get = src[name]
+        share = left // (len(src) - i)
+        idx = None
+        if nrows * row_bytes > share:
+            idx = np.sort(np.random.default_rng(seed).choice(nrows, share // (row_bytes + 8), replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), idx.astype(np.float64))
+            left -= 8 * len(idx)
+        a = get(idx)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        left -= a.nbytes
+
+
+def _whole(arrays):
+    """write_arrays entries of arrays held in host memory"""
+    return {k: (len(a), a[:1].nbytes, lambda idx, a=a: a if idx is None else a[idx]) for k, a in arrays.items()}
+
+
+def dump_outputs(out_dir, batch, budget=DUMP_BUDGET, seed=0):
+    """--dump-outputs of a batch workload: what a caller of the timed path reads back after a step, integers as float64
+    (exact), the visibility means V as float32: Batch.fetch_summary's result tables, the query identities and first-stage
+    cluster labels per row, V [row, frame], the match bit words, and `votes`, one row per voted (query, frame) tile:
+    [row, frame, points inside the frame, points per label 0 .. L-1]. Only entries the step writes are included, so two
+    runs with the same arguments give identical files."""
+    import numpy as np
+    import torch
+    descs = batch.host_descs
+    T, L = descs[0].T, descs[0].L
+    assert all(d.T == T and d.L == L for d in descs), "the batch workloads have one video shape"
+    summ = batch.fetch_summary()
+    ri = summ["rowinfo"]
+    ok = np.repeat(summ["vidinfo"][:, 1] > 0, [d.Nm for d in descs])
+    cand = np.nonzero((ri[:, 1] >= 0) & ok)[0]
+    n = (ri[cand, 3] - ri[cand, 2] + 1).astype(np.int64)
+    rows = np.repeat(cand, n)
+    frames = ri[rows, 2] + np.arange(len(rows)) - np.repeat(np.cumsum(n) - n, n)
+    f64 = lambda a: np.asarray(a, np.float64)
+
+    def votes(idx):
+        r, f = (rows, frames) if idx is None else (rows[idx], frames[idx])
+        rt, ft = torch.from_numpy(r).to(batch.device), torch.from_numpy(f.astype(np.int64)).to(batch.device)
+        hits = batch.hits.view(-1, T, L)[rt, ft].cpu().numpy()
+        uniq = batch.uniq.view(-1, T)[rt, ft].cpu().numpy()
+        return np.concatenate([f64(r)[:, None], f64(f)[:, None], f64(uniq)[:, None], f64(hits)], axis=1)
+
+    host = {k: f64(v) for k, v in summ.items()}
+    host.update(query_frame=f64(batch.qframe.cpu()), query_label=f64(batch.qlabel.cpu()), labels1=f64(batch.labels1.cpu()),
+                V=batch.V.view(-1, T).cpu().numpy(), match_bits=f64(batch.mbits.cpu().numpy().view(np.uint32)))
+    src = _whole(host)
+    src["votes"] = (len(rows), (3 + L) * 8, votes)
+    write_arrays(out_dir, src, budget, seed)
+
+
+def dump_list_results(out_dir, results):
+    """--dump-outputs of a list workload: the per-video results of the last timed pass, in list order, that the digest is
+    computed from: `videos` [frames, queries, candidates, status, clusters, keymasks, K2 tiles] and `digests`, the 32
+    bytes of each video's sha256 over its result tables (s2d_b200.workloads.video_digest), all as float64."""
+    import numpy as np
+    keys = ("frames", "queries", "candidates", "status", "clusters", "keymasks", "tiles")
+    videos = np.asarray([[r[k] for k in keys] for r in results], np.float64).reshape(-1, len(keys))
+    digests = np.asarray([list(bytes.fromhex(r["digest"])) for r in results], np.float64).reshape(-1, 32)
+    write_arrays(out_dir, _whole({"videos": videos, "digests": digests}))
+
+
 def list_specs(args):
     """the video list of a list workload (identical on every rank)"""
     from dataclasses import replace
@@ -440,7 +525,8 @@ def list_workload(args):
     homogeneous batch per GPU. The list is the same on every rank; s2d_b200.partition assigns videos to ranks (LPT over
     the byte cost), every rank runs its share through the device pipeline in HBM-sized chunks (device-timed), rank 0
     gathers the per-video results (timed) and hashes them: the digest must not depend on the number of GPUs.
-    Strong scaling: the total work is fixed."""
+    Strong scaling: the total work is fixed. --steps K times K passes over the list: every chunk of videos runs K times
+    on the device, the partition and the gather are done K times."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -527,27 +613,30 @@ def list_workload(args):
     local_stats = {}
 
     def worker(idx):
-        res, st, _ = runner.run_list([specs[i] for i in idx])
+        res, st, _ = runner.run_list([specs[i] for i in idx], reps=args.steps)
         local_stats.update(st)
         return res
 
     # the gather is timed on its own, after a barrier, so that it measures the exchange and not the ranks' drift
     parts = partition.lpt_partition(costs, world)
     t_part0 = time.perf_counter()
-    mine = partition.lpt_partition(costs, world)[rank]
+    for _ in range(args.steps):
+        mine = partition.lpt_partition(costs, world)[rank]
     t_part = time.perf_counter() - t_part0
     local = worker(mine)
     barrier()
-    if world > 1:
-        dist.barrier(group=host_pg)                   # host-side rendezvous right before the timed exchange
-    tg0 = time.perf_counter()
-    if world > 1:
-        gathered = [None] * world if rank == 0 else None
-        dist.gather_object(list(zip(mine, local)), gathered, dst=0, group=host_pg)
-        merged = sorted((p for part in gathered for p in part), key=lambda x: x[0]) if rank == 0 else None
-    else:
-        merged = sorted(zip(mine, local), key=lambda x: x[0])
-    t_gather = time.perf_counter() - tg0
+    t_gather = 0.0
+    for _ in range(args.steps):
+        if world > 1:
+            dist.barrier(group=host_pg)               # host-side rendezvous right before the timed exchange
+        tg0 = time.perf_counter()
+        if world > 1:
+            gathered = [None] * world if rank == 0 else None
+            dist.gather_object(list(zip(mine, local)), gathered, dst=0, group=host_pg)
+            merged = sorted((p for part in gathered for p in part), key=lambda x: x[0]) if rank == 0 else None
+        else:
+            merged = sorted(zip(mine, local), key=lambda x: x[0])
+        t_gather += time.perf_counter() - tg0
     clk = clocks.stop()
     dev_ms = max_over_ranks(local_stats["device_ms"])
     sum_ms = torch.tensor([local_stats["device_ms"], local_stats["k2_ms"], float(local_stats["k2_bytes"]), float(local_stats["k2_tiles"]),
@@ -559,6 +648,8 @@ def list_workload(args):
         results = [r for _, r in merged]
         assert [i for i, _ in merged] == list(range(len(specs)))
         digest = wl.list_digest(results)
+        if args.dump_outputs:
+            dump_list_results(args.dump_outputs, results)
         frames = sum(r["frames"] for r in results)
         total_s = dev_ms / 1000.0 + t_gather + t_part
         ref_digest, equal = None, None
@@ -577,8 +668,9 @@ def list_workload(args):
                 json.dump(dj, f, indent=1, sort_keys=True)
         loads = [sum(costs[i] for i in p) for p in parts]
         k2_gbs = tot[2] / (tot[1] / 1000.0) / 1e9 if tot[1] > 0 else 0.0
-        line = {"metric": METRIC, "value": frames / total_s, "unit": UNIT, "n_gpus": world, "steps": 1, "warmup": len(warm),
-                "ms_per_step": 1000 * total_s, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+        line = {"metric": METRIC, "value": frames * args.steps / total_s, "unit": UNIT, "n_gpus": world, "steps": args.steps,
+                "warmup": len(warm), "ms_per_step": 1000 * total_s / args.steps, "higher_is_better": True, "scaling": "strong",
+                "vs_baseline": None,
                 "dtype": "u8/int32 (f32 tracks, f64 scores)", "data": "synthetic",
                 "config": {"workload": f"{args.workload}: {LIST_WORKLOADS[args.workload]}", "videos": len(specs),
                            "frames": frames, "queries": sum(r["queries"] for r in results), "list_scale": args.list_scale,
@@ -586,8 +678,9 @@ def list_workload(args):
                            "partition": f"LPT by video over {world} GPU(s), host gather of per-video results (gather_object over gloo)",
                            "cache": "every chunk's inputs >> 126 MB L2, no flush needed"},
                 "timed_region": {"device_ms_max_over_ranks": dev_ms, "gather_ms": 1000 * t_gather, "partition_ms": 1000 * t_part,
-                                 "note": "device_ms = CUDA-event time of every chunk's kernels + result read-back, summed per rank, max over "
-                                         "ranks; generation of the synthetic inputs (upstream producers) is outside; gather timed after a barrier"},
+                                 "note": "device_ms = CUDA-event time of every chunk's kernels + result read-back, summed over chunks and "
+                                         "steps per rank, max over ranks; generation of the synthetic inputs (upstream producers) is outside; "
+                                         "gather and partition summed over steps, each gather timed after a barrier"},
                 "balance": {"max_over_mean_cost": max(loads) / (sum(loads) / len(loads)), "device_ms_sum_over_ranks": tot[0]},
                 "clocks": clk, "gpu_launches": int(tot[4]),
                 "roofline": {"kernel": "point_votes_tab_kernel (all chunks of all ranks)", "bound": "hbm", "achieved": k2_gbs, "peak": peak,
@@ -613,7 +706,8 @@ def list_workload(args):
 
 def c5_sweep(args, runner, rank, world, dev, barrier, max_over_ranks, clocks, peak, peak_src, all_cores, host_pg=None):
     """the 48 points of the sweep are dealt to the ranks round-robin by cost; per point: frames/s of the device path, the
-    K2 roofline fraction, and the CPU port on one query of the same video (all host cores / ranks per rank)."""
+    K2 roofline fraction, and the CPU port on one query of the same video (all host cores / ranks per rank). Every point's
+    videos run once untimed (it warms the shape), then --steps timed times."""
     import torch
     import torch.distributed as dist
     from s2d_b200 import partition
@@ -634,7 +728,7 @@ def c5_sweep(args, runner, rank, world, dev, barrier, max_over_ranks, clocks, pe
     threads = max(1, len(all_cores) // world)
     for pi in mine:
         M, P, Tw = pts[pi]
-        res, st, _ = runner.run_list(plists[pi], reps=2)      # second repetition is the one reported (first warms the shape)
+        res, st, _ = runner.run_list(plists[pi], reps=args.steps, warm=1)
         dev_ms += st["device_ms"]
         k2 = st["k2_bytes"] / (st["k2_ms"] / 1000.0) / 1e9 if st["k2_ms"] > 0 else 0.0
         rec = {"masks_per_frame": M, "tracks": P, "window": Tw, "videos": len(plists[pi]), "frames": st["frames"],
@@ -645,7 +739,7 @@ def c5_sweep(args, runner, rank, world, dev, barrier, max_over_ranks, clocks, pe
             fps, dt, npairs, n, Nm = cpu_sample_spec(plists[pi][0], 1, threads, dev)
             rec["cpu_frames_per_s"] = fps
             rec["cpu_sample"] = f"1 of {Nm} queries, {npairs} pairs in {dt:.2f} s on {threads} threads"
-        out.append((pi, rec))
+        out.append((pi, rec, res))
     barrier()
     clk = clocks.stop()
     if world > 1:
@@ -656,11 +750,13 @@ def c5_sweep(args, runner, rank, world, dev, barrier, max_over_ranks, clocks, pe
         merged = sorted(out, key=lambda x: x[0])
     t_max = max_over_ranks(dev_ms)
     if rank == 0:
-        recs = [r for _, r in merged]
+        recs = [r for _, r, _ in merged]
+        if args.dump_outputs:
+            dump_list_results(args.dump_outputs, [v for _, _, res in merged for v in res])
         frames = sum(r["frames"] for r in recs)
         fr = [r["k2_frac"] for r in recs]
-        line = {"metric": METRIC, "value": frames / (t_max / 1000.0), "unit": UNIT, "n_gpus": world, "steps": 1, "warmup": 3,
-                "ms_per_step": t_max, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+        line = {"metric": METRIC, "value": frames / (t_max / 1000.0), "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": 3,
+                "ms_per_step": t_max / args.steps, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": "u8/int32 (f32 tracks, f64 scores)", "data": "synthetic",
                 "config": {"workload": f"c5: {LIST_WORKLOADS['c5']}", "points": len(recs), "list_scale": args.list_scale,
                            "partition": f"LPT by sweep point over {world} GPU(s)", "cache": "inputs per point >> 126 MB L2"},
@@ -800,7 +896,7 @@ def run_e2e(args, vids, dev, world, params, barrier, binding):
     del src
     hv = [HostVideo(host[3 * i], host[3 * i + 1], host[3 * i + 2], vis_bits=bits, max_label=M) for i in range(npool)]
     pipe = HostPipeline(hv[:2 * chunk] if npool >= 2 * chunk else hv[:chunk], dev, params, chunk=chunk)
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     order = [hv[i % npool] for i in range(nvid)]
 
     pipe.run(order)                                   # warm-up (allocates the pinned result tables)

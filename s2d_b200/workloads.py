@@ -132,15 +132,17 @@ class DeviceRunner:
             out.append(cur)
         return out
 
-    def run_list(self, specs: Sequence[VideoSpec], reps: int = 1, keep_batch: bool = False):
-        """Returns (per-video results in list order, stats). stats: device_ms (sum over chunks of the event-timed
-        kernels + result read-back, per repetition), stage_ms, k2 bytes / tiles, frames, launches."""
+    def run_list(self, specs: Sequence[VideoSpec], reps: int = 1, keep_batch: bool = False, warm: int = 0):
+        """Every chunk of the list runs `warm` untimed repetitions, then `reps` timed ones. Returns (per-video results of
+        the last repetition in list order, stats). stats: device_ms (event-timed kernels + result read-back, summed over
+        chunks and timed repetitions), stage_ms, k2 bytes / tiles, frames and launches of all timed repetitions."""
         from .synth import make_scene_device
         dev = self.device
         results: List[Optional[dict]] = [None] * len(specs)
         stats = {"device_ms": 0.0, "frames": 0, "k2_bytes": 0, "k2_tiles": 0, "k2_ms": 0.0, "vis_bytes": 0, "vis_ms": 0.0,
                  "launches": 0, "chunks": 0, "stage_ms": {}}
         last = None
+        reps = max(1, reps)
         with torch.cuda.device(dev):
             for idx in self.chunks(specs):
                 scenes, vids = [], []
@@ -155,8 +157,8 @@ class DeviceRunner:
                 windowed = any(specs[i].window > 0 for i in idx)
                 host = {k: torch.empty(getattr(batch, k).shape, dtype=getattr(batch, k).dtype, pin_memory=True)
                         for k in ("vidinfo", "clusterinfo", "rowinfo", "glabel", "one2x")}
-                ms = 0.0
-                for rep in range(max(1, reps)):
+                ms, st = 0.0, {}
+                for rep in range(warm + reps):
                     timers = {}
                     ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
                     torch.cuda.synchronize(dev)
@@ -182,10 +184,12 @@ class DeviceRunner:
                         hbuf.copy_(getattr(batch, k), non_blocking=True)
                     ev[3].record()
                     ev[3].synchronize()
-                    ms = ev[0].elapsed_time(ev[1]) + ev[2].elapsed_time(ev[3])
-                    st = {k: sum(a.elapsed_time(b) for a, b in v) for k, v in timers.items()}
+                    if rep >= warm:
+                        ms += ev[0].elapsed_time(ev[1]) + ev[2].elapsed_time(ev[3])
+                        for k, v in timers.items():
+                            st[k] = st.get(k, 0.0) + sum(a.elapsed_time(b) for a, b in v)
                 stats["device_ms"] += ms
-                stats["launches"] += n1 + n2
+                stats["launches"] += (n1 + n2) * reps
                 stats["chunks"] += 1
                 for k, v in st.items():
                     stats["stage_ms"][k] = stats["stage_ms"].get(k, 0.0) + v
@@ -205,10 +209,10 @@ class DeviceRunner:
                     else:
                         lo, hi = rows[:, 2], rows[:, 3]
                     tiles = int((np.maximum(hi - lo + 1, 0) * cand).sum()) if ok else 0
-                    stats["k2_tiles"] += tiles
-                    stats["k2_bytes"] += 8 * s.P * tiles + s.T * s.H * s.W + 4 * (d.L + 1) * tiles
-                    stats["vis_bytes"] += d.Nm * d.T * ((((s.P + 31) // 32) * 4) if s.vis_bits else s.P) + 8 * d.Nm * d.T
-                    stats["frames"] += s.T
+                    stats["k2_tiles"] += tiles * reps
+                    stats["k2_bytes"] += (8 * s.P * tiles + s.T * s.H * s.W + 4 * (d.L + 1) * tiles) * reps
+                    stats["vis_bytes"] += (d.Nm * d.T * ((((s.P + 31) // 32) * 4) if s.vis_bits else s.P) + 8 * d.Nm * d.T) * reps
+                    stats["frames"] += s.T * reps
                     gl = summ["glabel"][d.row0:d.row0 + d.Nm]
                     results[i] = {"name": s.name, "frames": s.T, "queries": int(d.Nm), "candidates": int(cand.sum()),
                                   "status": int(summ["vidinfo"][j, 3]), "clusters": int(summ["vidinfo"][j, 0]),

@@ -1,4 +1,6 @@
 """CUDA path vs reference goldens and vs the CPU oracle, through the C ABI (needs a B200)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -93,14 +95,15 @@ def test_point_votes_all_pairs_vs_oracle(golden_case):
 
 
 @pytest.fixture(params=[0, 1, 2, 3, 4], ids=["product", "bitmap", "cta_per_tile", "table_any_P", "warp_any_frame"])
-def pv_variant(request):
-    """run a test once per point-votes kernel variant (include/s2d_b200.h: s2d_point_votes_variant)"""
+def pv_variant(request, monkeypatch):
+    """run a test once per point-votes kernel variant (include/s2d_b200.h: s2d_point_votes_variant); the superseded
+    bitmap kernel (1) only exists in the experiments build (make exp), which the runs of variant 1 load instead - also in a
+    debug run with S2D_B200_LIB pointing at the bounds-checked library, so those runs are not bounds-checked"""
     from s2d_b200 import _lib
-    try:
-        _lib.call("s2d_point_votes_variant", request.param)
-    except _lib.S2DError:
-        assert request.param == 1     # the superseded bitmap kernel only exists in the experiments build (make exp)
-        pytest.skip("variant 1 is compiled only into libs2d_b200_exp.so")
+    if request.param == 1:
+        monkeypatch.setattr(_lib, "LIB_PATH", os.path.join(os.path.dirname(_lib.LIB_PATH), "libs2d_b200_exp.so"))
+        monkeypatch.setattr(_lib, "_lib", None)
+    _lib.call("s2d_point_votes_variant", request.param)
     yield request.param
     _lib.call("s2d_point_votes_variant", 0)
 

@@ -39,7 +39,7 @@ def main():
         ref = None
         for cname, variant in configs:
             _lib.call("s2d_point_votes_variant", variant)
-            res, st, _ = runner.run_list(specs, reps=3)
+            res, st, _ = runner.run_list(specs, warm=2)
             dig = wl.list_digest(res)
             ref = ref or dig
             k2ms = st["k2_ms"]                                       # of the last repetition
