@@ -219,6 +219,34 @@ int s2d_rle_encode(const uint8_t* masks, int N, int H, int W, int max_runs, int3
 int s2d_rle_area_bbox(const int32_t* counts, const int64_t* offsets, int N, const int32_t* heights,
                       int32_t* area, int32_t* bbox, void* stream);
 
+/* Stage E on the device: COCO RLE of every keymask row straight from the label maps, without materialising a mask
+ * plane per keymask. Replaces the per-keymask mask_util.encode / toBbox of annotations.py:94-106 (maskApi.c rleEncode)
+ * for a whole batch. Row g = (frame, label) as K0 enumerates them in gid_of; only videos whose vidinfo[3] (final
+ * status) is 1 are encoded - the reference writes no annotation for the others, and their rows get no runs.
+ *   counts   int32, the rows' run lengths back to back: column-major, starting with a run of zeros (of length 0
+ *            when pixel (0, 0) is set), exactly what rleEncode produces for labels[f] == l
+ *   offsets  int64 [total_rows + 1]: row g's runs are counts[offsets[g] .. offsets[g + 1])
+ *   bbox     int32 [total_rows][4] = xmin, ymin, xmax, ymax (inclusive) of the mask; the area is K0's area[f][l]
+ *   needed   int64 [1] = offsets[total_rows], the counts the batch needs. Nothing is written at or past `capacity`;
+ *            when *needed > capacity the caller re-runs with a larger buffer (rows past the capacity are incomplete).
+ * Each frame's label bytes are read twice whatever the number of objects (a transition a -> b in column-major order is
+ * an edge of mask a and of mask b). Needs K0's gid_of and the final status of K4 (vidinfo) on the device: no host
+ * round trip, so the call can be captured in a CUDA graph. H * W < 2^31, H <= 65535. work: int32 scratch of
+ * s2d_label_rle_work_ints(total_frames, total_rows, max_H, max_W) elements. */
+int s2d_label_rle_work_ints(int64_t total_frames, int64_t total_rows, int max_H, int max_W, int64_t* out);
+int s2d_label_rle(const s2d_video_desc* descs, int nvideos, int max_T, int max_H, int max_W, int max_Nm,
+                  int64_t total_frames, int64_t total_rows, const int32_t* gid_of, const int32_t* vidinfo,
+                  int32_t* work, int64_t capacity, int32_t* counts, int64_t* offsets, int32_t* bbox,
+                  int64_t* needed, void* stream);
+
+/* COCO compressed-RLE strings of N run-length lists on the device (maskApi.c rleToString, as annotations.py:100 gets
+ * them through mask_util.encode): counts / offsets [N + 1] in the layout above (lists that end past `ncounts`, the
+ * valid length of counts, give empty strings). chars receives the strings back to back, str_offsets [N + 1] (int64)
+ * where each starts, *needed the total length; nothing is written at or past `capacity` (re-run when *needed >
+ * capacity). Byte-identical to the reference's packing. work: int32 scratch of N elements. */
+int s2d_rle_strings(const int32_t* counts, const int64_t* offsets, int N, int64_t ncounts, int32_t* work,
+                    int64_t capacity, char* chars, int64_t* str_offsets, int64_t* needed, void* stream);
+
 /* K4a. Scores and selection per candidate query: iou = hits/uniq (double), match bit when
  * iou > matching_threshold (cotracker_matching.py:710), one-to-many flag when >= one2x_frames
  * frames hold more than one mask with iou > one2x_iou (cotracker_matching.py:1082-1111).

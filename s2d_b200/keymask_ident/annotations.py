@@ -1,8 +1,9 @@
 """Drop-in for keymask_ident/annotations.py (stage E): single-video YTVIS json from the
 `cluster_*/group_*/frame{f}_mask{m}.png` tree. The reference calls pycocotools per keymask
 (mask_util.encode / area / toBbox, annotations.py:94-106); here all keymasks of a video are encoded
-in one batch on the GPU (s2d_rle_encode: column-major run lengths, area, bounding box) and only the
-base-48 string packing of the short count lists (maskApi.c rleToString) runs on the host.
+in one batch on the GPU (s2d_rle_encode: column-major run lengths, area, bounding box; s2d_rle_strings: the
+base-48 string packing of maskApi.c rleToString). Batched callers that got their annotations from
+s2d_b200.pipeline (stage E on the device) write the same json with write_video_annotations.
 pycocotools is not installable in the build container, so parity at the RLE boundary is pinned by
 the published algorithm and by decode round trips only (tests/test_dropin_gpu.py)."""
 from __future__ import annotations
@@ -23,7 +24,8 @@ except ImportError:
 
 
 class coco_rle:
-    """COCO compressed-RLE strings (maskApi.c rleToString / rleFrString) and the GPU batch encoder."""
+    """COCO compressed-RLE strings (maskApi.c rleToString / rleFrString) and the GPU batch encoder. to_string /
+    from_string are the host helpers; encode_batch packs on the device (s2d_rle_strings), byte for byte the same."""
 
     @staticmethod
     def to_string(cnts):
@@ -87,16 +89,47 @@ class coco_rle:
             if int(nr.max()) <= max_runs:
                 break
             max_runs = int(nr.max())                   # a mask with more runs than the first guess: once more
-        cn, ar, bb = counts.cpu().numpy(), area.cpu().numpy(), bbox.cpu().numpy()
+        # the masks' runs back to back, then the strings of all of them in one device pass
+        flat = counts[torch.arange(max_runs, device=dev)[None, :] < nruns[:, None].to(torch.int64)].contiguous()
+        offs = np.zeros(n + 1, np.int64)
+        offs[1:] = np.cumsum(nr.astype(np.int64))
+        strings = coco_rle.strings_device(flat, offs, dev)
+        ar, bb = area.cpu().numpy(), bbox.cpu().numpy()
         out = []
         for i in range(n):
-            rle = {"size": [int(h), int(w)], "counts": coco_rle.to_string(cn[i, :nr[i]].tolist())}
+            rle = {"size": [int(h), int(w)], "counts": strings[i]}
             if ar[i] == 0:
                 box = [0.0, 0.0, 0.0, 0.0]
             else:
                 box = [float(bb[i, 0]), float(bb[i, 1]), float(bb[i, 2] - bb[i, 0] + 1), float(bb[i, 3] - bb[i, 1] + 1)]
             out.append((rle, int(ar[i]), box))
         return out
+
+
+    @staticmethod
+    def strings_device(counts, offsets, dev):
+        """rleToString of N run-length lists on the device: counts (device int32, the lists back to back), offsets
+        (host int64 [N + 1]) -> list of N strings."""
+        from s2d_b200 import _lib
+        n = len(offsets) - 1
+        ncounts = int(offsets[-1])
+        st = torch.cuda.current_stream(dev).cuda_stream
+        d_off = torch.from_numpy(np.ascontiguousarray(offsets, np.int64)).to(dev)
+        work = torch.empty(n, dtype=torch.int32, device=dev)
+        soff = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        need = torch.zeros(1, dtype=torch.int64, device=dev)
+        cap = 2 * ncounts + 16                      # most runs of a keymask take one or two characters
+        while True:
+            chars = torch.empty(cap, dtype=torch.uint8, device=dev)
+            _lib.call("s2d_rle_strings", counts.data_ptr(), d_off.data_ptr(), n, ncounts, work.data_ptr(), cap,
+                      chars.data_ptr(), soff.data_ptr(), need.data_ptr(), st)
+            total = int(need.item())
+            if total <= cap:
+                break
+            cap = total
+        text = chars[:max(1, total)].cpu().numpy().tobytes()[:total].decode("ascii")
+        so = soff.cpu().numpy()
+        return [text[so[i]:so[i + 1]] for i in range(n)]
 
 
 def rle_area_bbox_batch(rles):
@@ -126,24 +159,53 @@ def rle_area_bbox_batch(rles):
     return [(int(a[i]), [float(v) for v in b[i]]) for i in range(len(rles))]
 
 
-def write_annotation_for_video(video_path, cluster_masks_path, annotation_output_path, visibility_data):
-    """Same contract as the reference (annotations.py:8-140)."""
+def _video_entry(video_path):
+    """The `videos` entry the reference builds from the video's image folder (annotations.py:13-40), None without
+    images."""
     video_name = os.path.basename(video_path)
     video_files = sorted(f for f in os.listdir(video_path) if f.endswith((".jpg", ".png", ".jpeg")))
     if not video_files:
         print(f"No image files found in {video_path}")
-        return
+        return None
     with Image.open(os.path.join(video_path, video_files[0])) as img:
         width, height = img.size
-    video = {"license": 1, "coco_url": "", "height": height, "width": width, "length": len(video_files),
-             "date_captured": "2019-04-11 00:55:41.903902",
-             "file_names": [os.path.join(video_name, f) for f in video_files], "flickr_url": "", "id": 1}
+    return {"license": 1, "coco_url": "", "height": height, "width": width, "length": len(video_files),
+            "date_captured": "2019-04-11 00:55:41.903902",
+            "file_names": [os.path.join(video_name, f) for f in video_files], "flickr_url": "", "id": 1}
+
+
+def _dump_video_json(video, annotations, annotation_output_path, video_path):
+    """`{videos, annotations, categories}` of one video to <annotation_output_path>/<video name>.json
+    (annotations.py:131-140)."""
+    os.makedirs(annotation_output_path, exist_ok=True)
+    with open(os.path.join(annotation_output_path, f"{os.path.basename(video_path)}.json"), "w") as f:
+        json.dump({"videos": [video], "annotations": annotations,
+                   "categories": [{"supercategory": "object", "id": 1, "name": "fg"}]}, f)
+
+
+def write_video_annotations(video_path, annotations, annotation_output_path):
+    """The json write_annotation_for_video produces, for annotations computed elsewhere - the device stage E of the
+    batched path (s2d_b200.pipeline: Batch.annotations, discover_keymasks(..., annotations=True)). Nothing is written
+    for a video without annotations (None: the reference writes no json for a failed video) or without images."""
+    if annotations is None:
+        return
+    video = _video_entry(video_path)
+    if video is not None:
+        _dump_video_json(video, annotations, annotation_output_path, video_path)
+
+
+def write_annotation_for_video(video_path, cluster_masks_path, annotation_output_path, visibility_data):
+    """Same contract as the reference (annotations.py:8-140)."""
+    video = _video_entry(video_path)
+    if video is None:
+        return
+    height, width = video["height"], video["width"]
     cluster_dirs = sorted(d for d in os.listdir(cluster_masks_path)
                           if os.path.isdir(os.path.join(cluster_masks_path, d)) and d.startswith("cluster_")
                           and any(f.endswith(".png") for f in os.listdir(os.path.join(cluster_masks_path, d))))
     with open(os.path.join(cluster_masks_path, "video_one2x_data.json")) as f:
         one2x_data = json.load(f)
-    annotations, ann_id, n = [], 1, len(video_files)
+    annotations, ann_id, n = [], 1, video["length"]
     pending = []
     for cname in cluster_dirs:
         cdir = os.path.join(cluster_masks_path, cname)
@@ -178,7 +240,4 @@ def write_annotation_for_video(video_path, cluster_masks_path, annotation_output
         enc = coco_rle.encode_batch(np.stack([it[4] for it in items]))
         for (segs, areas, boxes, fidx, _), (rle, area, box) in zip(items, enc):
             segs[fidx], areas[fidx], boxes[fidx] = rle, area, box
-    os.makedirs(annotation_output_path, exist_ok=True)
-    with open(os.path.join(annotation_output_path, f"{video_name}.json"), "w") as f:
-        json.dump({"videos": [video], "annotations": annotations,
-                   "categories": [{"supercategory": "object", "id": 1, "name": "fg"}]}, f)
+    _dump_video_json(video, annotations, annotation_output_path, video_path)

@@ -201,6 +201,25 @@ class Batch:
                 self.gram_off = torch.tensor(offs, dtype=torch.int64, device=dev)
                 self.gram_planes = torch.empty(pmax, dtype=torch.uint8, device=dev)
                 self._gram_videos = [(i, offs[i]) for i in big]
+        # stage E: COCO RLE of every keymask row from the label maps (counts, offsets, boxes) and its strings
+        self.rle_work = self.rle_counts = self.rle_off = self.rle_bbox = self.rle_need = None
+        self.str_work = self.str_off = self.rle_chars = None
+        self.rle_cap = self.str_cap = 0
+        if "E" in st:
+            assert "L" in st and "D" in st, 'stage "E" reads K0\'s gid_of ("L") and the final status of K4 ("D")'
+            self.max_H = max(descs[i].H for i in range(nv))
+            self.max_W = max(descs[i].W for i in range(nv))
+            _lib.call("s2d_label_rle_work_ints", frame0, row0, self.max_H, self.max_W, C.byref(n))
+            self.rle_work = z(n.value)
+            self.rle_off = torch.empty(row0 + 1, dtype=torch.int64, device=dev)
+            self.rle_bbox = z(4 * row0)
+            self.rle_need = torch.zeros(2, dtype=torch.int64, device=dev)    # counts, string bytes the run needed
+            self.str_work = z(row0)
+            self.str_off = torch.empty(row0 + 1, dtype=torch.int64, device=dev)
+            # first guess: blob-like maps have about two edges per (object, column); too small re-runs (annotations())
+            cap = sum(descs[i].T * 8 * descs[i].W for i in range(nv)) + 2 * row0
+            self._alloc_rle(cap, 3 * cap)
+        self._graph = None
         self.kernel_launches_per_run = 0
         # persistent TMA-fed votes kernel (the library falls back by itself when P is odd)
         self.use_tma = bool(persistent_votes)
@@ -266,8 +285,19 @@ class Batch:
             call("group", 8, "s2d_group_gram", d, nv, self.max_Nm, self.max_NW, self.total_rows, p(self.mbits),
                  p(self.rowinfo), p(self.one2x), p(self.grpwork), p(self.glabel), p(self.grp_n),
                  p(self.grp_one2x), p(self.vidinfo), p(self.clusterinfo), p(self.gram), p(self.gram_off), st)
+        if "E" in stages:
+            call("label_rle", 5, "s2d_label_rle", d, nv, self.max_T, self.max_H, self.max_W, self.max_Nm,
+                 self.total_frames, self.total_rows, p(self.gid_of), p(self.vidinfo), p(self.rle_work), self.rle_cap,
+                 p(self.rle_counts), p(self.rle_off), p(self.rle_bbox), p(self.rle_need), st)
+            call("rle_strings", 3, "s2d_rle_strings", p(self.rle_counts), p(self.rle_off), self.total_rows, self.rle_cap,
+                 p(self.str_work), self.str_cap, p(self.rle_chars), p(self.str_off), p(self.rle_need) + 8, st)
         self.kernel_launches_per_run = launches
         return launches
+
+    def _alloc_rle(self, counts_cap: int, chars_cap: int):
+        self.rle_cap, self.str_cap = int(counts_cap), int(chars_cap)
+        self.rle_counts = torch.empty(max(1, self.rle_cap), dtype=torch.int32, device=self.device)
+        self.rle_chars = torch.empty(max(1, self.str_cap), dtype=torch.uint8, device=self.device)
 
     def capture(self, params: Params = Params(), stages: Optional[str] = None):
         """Record the whole path of this batch once as a CUDA graph; replay() then costs one launch
@@ -281,6 +311,7 @@ class Batch:
             with torch.cuda.graph(g):
                 self.run(params, stages=stages)
         self._graph = g
+        self._graph_args = (params, stages)
         return g
 
     def replay(self):
@@ -447,6 +478,79 @@ class Batch:
         return results
 
 
+    def rle_tables(self, counts: bool = False):
+        """Host copy of stage E's device tables after run() / replay(): per row (global id) `offsets` of its runs,
+        `bbox` (xmin, ymin, xmax, ymax), `str_off` of its string in `chars`; `counts` (the runs) on request. When a
+        buffer was too small for this batch (the device reports what it needed; noise-like label maps have about two
+        edges per pixel) it is grown and stage E re-run - its inputs are still in place - and a captured graph is
+        recorded again on the new buffers."""
+        assert "E" in self.stages, 'stage-E tables need a batch built with stage "E"'
+        with torch.cuda.device(self.device):
+            torch.cuda.synchronize(self.device)
+            need = self.rle_need.cpu().tolist()
+            if need[0] > self.rle_cap or need[1] > self.str_cap:
+                # once the counts fit, the string size the device reports is exact
+                while need[0] > self.rle_cap or need[1] > self.str_cap:
+                    self._alloc_rle(max(need[0], self.rle_cap), max(need[1], self.str_cap))
+                    self.run(stages="E")
+                    torch.cuda.synchronize(self.device)
+                    need = self.rle_need.cpu().tolist()
+                if self._graph is not None:
+                    self.capture(*self._graph_args)
+                    torch.cuda.synchronize(self.device)
+            out = {"offsets": self.rle_off.cpu().numpy(), "bbox": self.rle_bbox.cpu().numpy().reshape(-1, 4),
+                   "str_off": self.str_off.cpu().numpy(),
+                   "chars": self.rle_chars[:max(1, need[1])].cpu().numpy().tobytes()[:need[1]].decode("ascii")}
+            if counts:
+                out["counts"] = self.rle_counts[:max(1, need[0])].cpu().numpy()[:need[0]]
+        return out
+
+    def annotations(self, results=None):
+        """Stage E: per video the `annotations` list of the YTVIS json the reference writes for it
+        (keymask_ident/annotations.py:8-140), or None when the video's final status is not 1 (the reference writes
+        none). Needs a batch built with "E" in its stages, after run() or replay(). `results`: this step's decode(),
+        when the caller has it already.
+
+        Built from decode()'s clusters, groupings and one2x and the device RLE tables, in the reference's order:
+        cluster directories with candidates in lexicographic order of `cluster_{c}`, groups in lexicographic order
+        of `group_{l}`, ids from 1 across the video. A group with two members on one frame keeps the member with the
+        largest label id (the reference keeps whichever PNG its directory listing returns last)."""
+        tab = self.rle_tables()
+        res = results if results is not None else self.decode(want_comps=False)
+        soff, chars, bbox = tab["str_off"], tab["chars"], tab["bbox"]
+        area = self.area.cpu().numpy().reshape(-1, S2D_MAX_LABELS)
+        gid_of = self.gid_of.cpu().numpy().reshape(-1, S2D_MAX_LABELS)
+        out = []
+        for vi, r in enumerate(res):
+            if r["status"] != 1:
+                out.append(None)
+                continue
+            d = self.host_descs[vi]
+            T, H, W, f0, r0 = d.T, d.H, d.W, d.frame0, d.row0
+            with_cands = [c for c, cl in enumerate(r["clusters"]) if any(x["candidates"] for x in cl["all_candidates"])]
+            groups_of = {gr["cluster_id"]: gr["overall_mask_ids_per_label"] for gr in r["groupings"]}
+            anns = []
+            for c in sorted(with_cands, key=lambda c: f"cluster_{c}"):
+                cname = f"cluster_{c}"
+                if cname not in r["one2x"]:
+                    continue
+                groups = groups_of.get(c, {})
+                for lab in sorted(groups, key=lambda l: f"group_{l}"):
+                    segs, boxes, areas = [None] * T, [None] * T, [None] * T
+                    for f, m in sorted(groups[lab], key=lambda fm: fm[1]):      # tie rule: the largest label id wins
+                        g = r0 + int(gid_of[f0 + f, m])
+                        segs[f] = {"size": [H, W], "counts": chars[soff[g]:soff[g + 1]]}
+                        x0, y0, x1, y1 = (int(v) for v in bbox[g])
+                        boxes[f] = [float(x0), float(y0), float(x1 - x0 + 1), float(y1 - y0 + 1)]
+                        areas[f] = int(area[f0 + f, m])
+                    anns.append({"video_id": 1, "iscrowd": 0, "height": H, "width": W, "length": T,
+                                 "segmentations": segs, "bboxes": boxes, "areas": areas, "category_id": 1,
+                                 "id": len(anns) + 1, "one2x": round(float(r["one2x"][cname][f"group_{lab}"]["avg_one2x"]), 2),
+                                 "visibility_ranges": [list(x) for x in r["clusters"][c]["ranges"]]})
+            out.append(anns)
+        return out
+
+
 def pack_vis_bits(vis: torch.Tensor) -> torch.Tensor:
     """[Nm,T,P] visibility flags (bool / u8) -> int32 [Nm,T,ceil(P/32)] words, bit p % 32 of word p // 32 = flag p: the
     producer-side wire format of S2D_DESC_VIS_BITS (torch plumbing; one pass over the flags where they are born)."""
@@ -473,10 +577,17 @@ def _setbits(words: np.ndarray, limit: int):
     return out
 
 
-def discover_keymasks(videos: List[VideoInput], params: Params = Params(), want_comps: bool = True):
+def discover_keymasks(videos: List[VideoInput], params: Params = Params(), want_comps: bool = True,
+                      annotations: bool = False):
     """Public in-memory entry point: run stages A-D for a batch of videos on their device and
-    return one result dict per video."""
-    b = Batch(videos)
+    return one result dict per video. annotations=True runs stage E as well: each dict gains "annotations", the
+    YTVIS annotation list the reference writes for the video (None when its status is not 1; see
+    Batch.annotations and keymask_ident.annotations.write_video_annotations)."""
+    b = Batch(videos, stages="LVBDE" if annotations else "LVBD")
     b.run(params)
     torch.cuda.synchronize(b.device)
-    return b.decode(want_comps=want_comps)
+    res = b.decode(want_comps=want_comps)
+    if annotations:
+        for r, a in zip(res, b.annotations(res)):
+            r["annotations"] = a
+    return res
