@@ -247,6 +247,40 @@ int s2d_label_rle(const s2d_video_desc* descs, int nvideos, int max_T, int max_H
 int s2d_rle_strings(const int32_t* counts, const int64_t* offsets, int N, int64_t ncounts, int32_t* work,
                     int64_t capacity, char* chars, int64_t* str_offsets, int64_t* needed, void* stream);
 
+/* Annotation layout of stage E: which keymask rows become which YTVIS annotation, in the reference's order
+ * (annotations.py:8-140 walks `cluster_*` and `group_*` directories sorted as strings), as compact tables. Reads the
+ * tables of stages L, B, D and E already on the device; only videos whose vidinfo[3] (final status) is 1 get entries.
+ *   - a cluster c (< S2D_MAX_CLUSTERS) counts when one of its rows (rowinfo.x == c) is the candidate of a run r: rowinfo.y
+ *     == r, r below the cluster's number of runs and winner bit r of the row set. Counted clusters are ordered as the
+ *     strings cluster_{c};
+ *   - its groups are the distinct glabel >= 0 of its rows, ordered as the strings group_{l} (group_10 before group_2);
+ *     one annotation per group, numbered from 1 across the video;
+ *   - the members of a group are its rows; of two on one frame the one with the larger label id is kept.
+ * Outputs (caller-sized from host numbers; A <= total_rows annotations, M <= total_rows members, S <= the string bytes
+ * s2d_rle_strings reported, K <= S2D_MAX_CLUSTERS * nvideos clusters, R <= S2D_MAX_CLUSTERS / 2 * (total_frames +
+ * nvideos) range pairs; sizes int64 [5] receives A, M, S, K, R):
+ *   vann        int32 [nvideos][2]  number of annotations of the video, index of its first
+ *   ann         int32 [A][7]        cluster c, group l, grp_n and grp_one2x of (c, l) (the host divides them), index of the
+ *                                   cluster's range list in `clusters`, first member, number of members
+ *   members     int32 [M][6]        frame, bbox (xmin, ymin, xmax, ymax), area;  member_off int64 [M]: start of the member's
+ *                                   string in `chars` (it ends where the next member's starts, the last at S)
+ *   chars       the members' strings back to back, in (video, annotation, frame) order; nothing is written at or past
+ *               `capacity`, and a string that does not lie inside rle_chars [0, nchars) is not copied (when stage E's
+ *               own capacities were short the caller re-runs stage E and this call)
+ *   clusters    int32 [K][2]        first pair in `pairs`, number of pairs: [start, end] of every visibility run
+ *   pairs       int32 [R][2]
+ * The host only slices: no decision per row is left to it. rle_bbox / str_off / rle_chars as s2d_label_rle and
+ * s2d_rle_strings left them, area / gid_of of K0. No host round trip: the call can be captured in a CUDA graph.
+ * work: int32 scratch of s2d_annotation_layout_work_ints(total_rows, nvideos) elements, 8-byte aligned. */
+int s2d_annotation_layout_work_ints(int64_t total_rows, int nvideos, int64_t* out);
+int s2d_annotation_layout(const s2d_video_desc* descs, int nvideos, int64_t total_rows, const int32_t* vidinfo,
+                          const int32_t* rowinfo, const uint32_t* winbits, const uint32_t* rsbits, const uint32_t* rebits,
+                          const int32_t* glabel, const int32_t* qframe, const int32_t* qlabel, const int32_t* grp_n,
+                          const int32_t* grp_one2x, const int32_t* area, const int32_t* gid_of, const int32_t* rle_bbox,
+                          const int64_t* str_off, const char* rle_chars, int64_t nchars, int32_t* work, int32_t* vann,
+                          int32_t* ann, int32_t* members, int64_t* member_off, int32_t* clusters, int32_t* pairs,
+                          int64_t capacity, char* chars, int64_t* sizes, void* stream);
+
 /* K4a. Scores and selection per candidate query: iou = hits/uniq (double), match bit when
  * iou > matching_threshold (cotracker_matching.py:710), one-to-many flag when >= one2x_frames
  * frames hold more than one mask with iou > one2x_iou (cotracker_matching.py:1082-1111).

@@ -14,7 +14,8 @@ from typing import List, Optional, Sequence
 
 import torch
 
-from .pipeline import Batch, Params, VideoInput
+from ._lib import S2D_VIDINFO_WORDS
+from .pipeline import LAYOUT_TABLES, Batch, Params, VideoInput, annotations_from_layout
 
 
 @dataclass
@@ -37,14 +38,22 @@ class HostVideo:
 class HostPipeline:
     """Two staging sets + batches for chunks of `chunk` videos. `like` gives the shapes of the slots: `chunk` entries
     (both sets alike) or 2 * `chunk` entries (even chunks land in the first half's shapes, odd chunks in the second
-    half's). The allocation happens here, once; run() only enqueues copies and kernels."""
+    half's). The allocation happens here, once; run() only enqueues copies and kernels.
+
+    `annotations=True` adds stage E and its annotation layout (Batch.layout) to every chunk, and run() gives each
+    video's YTVIS annotation list as well. Before a staging set is reused, the host reads the stage-E needs and layout
+    sizes of the chunk it holds (the next chunk's copies are in flight meanwhile): a short capacity is grown and stage
+    E and the layout re-run on that set, whose label maps are still staged; then only the used part of the layout
+    tables is copied back."""
 
     RESULT_TABLES = ("vidinfo", "clusterinfo", "rowinfo", "glabel", "one2x")
 
-    def __init__(self, like: Sequence[HostVideo], device, params: Params = Params(), chunk: Optional[int] = None):
+    def __init__(self, like: Sequence[HostVideo], device, params: Params = Params(), chunk: Optional[int] = None,
+                 annotations: bool = False):
         self.device = torch.device(device)
         self.params = params
         self.chunk = int(chunk) if chunk else len(like)
+        self.annotations = bool(annotations)
         assert len(like) in (self.chunk, 2 * self.chunk)
         halves = [list(like[:self.chunk]), list(like[-self.chunk:])]
         self.sigs = [[v.signature() for v in h] for h in halves]
@@ -55,31 +64,42 @@ class HostPipeline:
                                  torch.empty(v.tracks.shape, dtype=torch.float32, device=self.device),
                                  torch.empty(v.vis.shape, dtype=v.vis.dtype, device=self.device),
                                  vis_bits=v.vis_bits, max_label=v.max_label) for v in h]
-                b = Batch(dv, device=self.device)
+                b = Batch(dv, device=self.device, stages="LVBDE" if self.annotations else "LVBD")
                 self.sets.append((dv, b))
             self.copy_streams = [torch.cuda.Stream(self.device), torch.cuda.Stream(self.device)]
             self.compute_stream = torch.cuda.Stream(self.device)
         self.host_results: List[dict] = []          # one set of pinned result tables per chunk, grown on first use
+        self.host_sizes: List[torch.Tensor] = []    # annotations: per chunk stage E's need (2) and the layout sizes (5)
+        self.host_layout: List[dict] = []           # annotations: per chunk pinned layout tables, grown on demand
         self.h2d_bytes = 0
         self.d2h_bytes = 0
         self.launches = 0
+        self.reruns = 0
 
     def run(self, videos: Sequence[HostVideo]) -> List[dict]:
         """All videos, chunk by chunk. Returns one dict of pinned host result tables per chunk (owned by the pipeline,
-        overwritten by the next run). Synchronises the device once, at the end."""
+        overwritten by the next run); with annotations=True each dict also holds "annotations": per video of the chunk,
+        in list order, its annotation list (keymask_ident.annotations.write_video_annotations) or None when its status
+        is not 1. Synchronises the device once at the end, and with annotations twice per chunk as well."""
         assert len(videos) % self.chunk == 0, "the list must be a whole number of chunks"
         nchunks = len(videos) // self.chunk
         while len(self.host_results) < nchunks:      # first call only: pinned result tables for every chunk
             b0 = self.sets[len(self.host_results) % 2][1]
             self.host_results.append({k: torch.empty(getattr(b0, k).shape, dtype=getattr(b0, k).dtype, pin_memory=True)
                                       for k in self.RESULT_TABLES})
+            if self.annotations:
+                self.host_sizes.append(torch.empty(7, dtype=torch.int64, pin_memory=True))
+                self.host_layout.append({})
         done = [None, None]
-        self.h2d_bytes = self.d2h_bytes = self.launches = 0
+        self.h2d_bytes = self.d2h_bytes = self.launches = self.reruns = 0
         with torch.cuda.device(self.device):
             for c in range(nchunks):
                 s = c % 2
                 dv, b = self.sets[s]
+                copied = None
                 if done[s] is not None:
+                    if self.annotations:
+                        copied = self._collect(c - 2, done[s])    # chunk c - 2 is complete before its set is reused
                     self.copy_streams[s].wait_event(done[s])          # staging set s is free again
                 with torch.cuda.stream(self.copy_streams[s]):
                     for j in range(self.chunk):
@@ -94,10 +114,63 @@ class HostPipeline:
                 self.compute_stream.wait_event(ready)
                 with torch.cuda.stream(self.compute_stream):
                     self.launches += b.run(self.params)
-                    for k, hbuf in self.host_results[c].items():
+                    if self.annotations:
+                        self.launches += b.layout()
+                        self._copy_sizes(c, b)
+                    for k in self.RESULT_TABLES:
+                        hbuf = self.host_results[c][k]
                         hbuf.copy_(getattr(b, k), non_blocking=True)
                         self.d2h_bytes += hbuf.numel() * hbuf.element_size()
                     done[s] = torch.cuda.Event()
                     done[s].record()
+                if copied is not None:
+                    # chunk c's copies and step are enqueued: the DMA stays busy while chunk c - 2's json objects are built
+                    copied.synchronize()
+                    self._assemble(c - 2)
+            if self.annotations:
+                for c in range(max(0, nchunks - 2), nchunks):
+                    self._collect(c, done[c % 2]).synchronize()
+                    self._assemble(c)
             self.compute_stream.synchronize()
         return self.host_results[:nchunks]
+
+    def _assemble(self, c):
+        """chunk c's annotation lists from its pinned layout tables (copied back already)"""
+        b = self.sets[c % 2][1]
+        hs = self.host_sizes[c].tolist()
+        n = {k: w * int(hs[2 + i]) for k, (w, i) in LAYOUT_TABLES.items()}
+        n["vann"] = 2 * b.nv
+        tabs = {k: t[:n[k]].numpy() for k, t in self.host_layout[c].items()}
+        status = self.host_results[c]["vidinfo"].numpy()[3::S2D_VIDINFO_WORDS]
+        self.host_results[c]["annotations"] = annotations_from_layout(b.host_descs, status, tabs)
+
+    def _copy_sizes(self, c, b):
+        hs = self.host_sizes[c]
+        hs[:2].copy_(b.rle_need, non_blocking=True)
+        hs[2:].copy_(b.al_sizes, non_blocking=True)
+        self.d2h_bytes += hs.numel() * hs.element_size()
+
+    def _collect(self, c, done):
+        """Chunk c's annotations: wait for its step, grow and re-run stage E and the layout on its set while a capacity
+        was short, then copy the used part of the layout tables to pinned host buffers. Enqueued on the set's copy
+        stream, so the set's next host -> device copies follow it. Returns an event recorded after the copies."""
+        b = self.sets[c % 2][1]
+        st = self.copy_streams[c % 2]
+        done.synchronize()
+        hs = self.host_sizes[c]
+        with torch.cuda.stream(st):
+            while not b.rle_fits(hs[:2].tolist()):
+                b.grow_rle(hs[:2].tolist())
+                self.launches += b.run(self.params, stages="E") + b.layout()
+                self.reruns += 1
+                self._copy_sizes(c, b)
+                st.synchronize()
+            hl = self.host_layout[c]
+            for k, t in b.layout_views(hs[2:].tolist()).items():
+                if k not in hl or hl[k].numel() < t.numel():
+                    hl[k] = torch.empty(t.numel() + t.numel() // 4 + 64, dtype=t.dtype, pin_memory=True)
+                hl[k][:t.numel()].copy_(t, non_blocking=True)
+                self.d2h_bytes += t.numel() * t.element_size()
+            copied = torch.cuda.Event()
+            copied.record()
+        return copied

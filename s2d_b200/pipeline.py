@@ -203,7 +203,7 @@ class Batch:
                 self._gram_videos = [(i, offs[i]) for i in big]
         # stage E: COCO RLE of every keymask row from the label maps (counts, offsets, boxes) and its strings
         self.rle_work = self.rle_counts = self.rle_off = self.rle_bbox = self.rle_need = None
-        self.str_work = self.str_off = self.rle_chars = None
+        self.str_work = self.str_off = self.rle_chars = self.al_work = self.al_chars = None
         self.rle_cap = self.str_cap = 0
         if "E" in st:
             assert "L" in st and "D" in st, 'stage "E" reads K0\'s gid_of ("L") and the final status of K4 ("D")'
@@ -216,6 +216,17 @@ class Batch:
             self.rle_need = torch.zeros(2, dtype=torch.int64, device=dev)    # counts, string bytes the run needed
             self.str_work = z(row0)
             self.str_off = torch.empty(row0 + 1, dtype=torch.int64, device=dev)
+            # annotation layout (s2d_annotation_layout): annotations and members number at most one per row, the
+            # packed strings at most stage E's, clusters S2D_MAX_CLUSTERS and runs ceil(T / 2) per cluster per video
+            _lib.call("s2d_annotation_layout_work_ints", row0, nv, C.byref(n))
+            self.al_work = z(n.value)
+            self.al_vann = z(2 * nv)
+            self.al_ann = z(7 * row0)
+            self.al_members = z(6 * row0)
+            self.al_member_off = torch.empty(row0, dtype=torch.int64, device=dev)
+            self.al_clusters = z(2 * S2D_MAX_CLUSTERS * nv)
+            self.al_pairs = z(2 * (S2D_MAX_CLUSTERS // 2) * (frame0 + nv))
+            self.al_sizes = torch.zeros(5, dtype=torch.int64, device=dev)     # annotations, members, string bytes, clusters, pairs
             # first guess: blob-like maps have about two edges per (object, column); too small re-runs (annotations())
             cap = sum(descs[i].T * 8 * descs[i].W for i in range(nv)) + 2 * row0
             self._alloc_rle(cap, 3 * cap)
@@ -298,6 +309,7 @@ class Batch:
         self.rle_cap, self.str_cap = int(counts_cap), int(chars_cap)
         self.rle_counts = torch.empty(max(1, self.rle_cap), dtype=torch.int32, device=self.device)
         self.rle_chars = torch.empty(max(1, self.str_cap), dtype=torch.uint8, device=self.device)
+        self.al_chars = torch.empty(max(1, self.str_cap), dtype=torch.uint8, device=self.device)
 
     def capture(self, params: Params = Params(), stages: Optional[str] = None):
         """Record the whole path of this batch once as a CUDA graph; replay() then costs one launch
@@ -486,18 +498,7 @@ class Batch:
         recorded again on the new buffers."""
         assert "E" in self.stages, 'stage-E tables need a batch built with stage "E"'
         with torch.cuda.device(self.device):
-            torch.cuda.synchronize(self.device)
-            need = self.rle_need.cpu().tolist()
-            if need[0] > self.rle_cap or need[1] > self.str_cap:
-                # once the counts fit, the string size the device reports is exact
-                while need[0] > self.rle_cap or need[1] > self.str_cap:
-                    self._alloc_rle(max(need[0], self.rle_cap), max(need[1], self.str_cap))
-                    self.run(stages="E")
-                    torch.cuda.synchronize(self.device)
-                    need = self.rle_need.cpu().tolist()
-                if self._graph is not None:
-                    self.capture(*self._graph_args)
-                    torch.cuda.synchronize(self.device)
+            need = self._settle_rle()
             out = {"offsets": self.rle_off.cpu().numpy(), "bbox": self.rle_bbox.cpu().numpy().reshape(-1, 4),
                    "str_off": self.str_off.cpu().numpy(),
                    "chars": self.rle_chars[:max(1, need[1])].cpu().numpy().tobytes()[:need[1]].decode("ascii")}
@@ -505,50 +506,111 @@ class Batch:
                 out["counts"] = self.rle_counts[:max(1, need[0])].cpu().numpy()[:need[0]]
         return out
 
+    def _settle_rle(self):
+        """Wait for the step, and grow the stage-E buffers and re-run stage E (re-recording a captured graph) while
+        the device reports that a capacity was short. Returns the final `need` (counts, string bytes)."""
+        torch.cuda.synchronize(self.device)
+        need = self.rle_need.cpu().tolist()
+        if self.rle_fits(need):
+            return need
+        while not self.rle_fits(need):
+            self.grow_rle(need)
+            self.run(stages="E")
+            torch.cuda.synchronize(self.device)
+            need = self.rle_need.cpu().tolist()
+        if self._graph is not None:
+            self.capture(*self._graph_args)
+            torch.cuda.synchronize(self.device)
+        return need
+
+    def rle_fits(self, need) -> bool:
+        """Whether stage E's tables are complete, given a host copy of `rle_need`."""
+        return need[0] <= self.rle_cap and need[1] <= self.str_cap
+
+    def grow_rle(self, need):
+        """Grow the stage-E buffers (and the layout's string buffer) to a host copy of `rle_need`; stage E has to be
+        run again. Once the counts fit, the string size the device reports is exact, so at most two rounds are needed."""
+        self._alloc_rle(max(need[0], self.rle_cap), max(need[1], self.str_cap))
+
+    def layout(self, stream=None) -> int:
+        """Enqueue the annotation layout (s2d_annotation_layout) of this step's stage-E tables on `stream` (default:
+        torch's current stream): per video the annotations, their members and strings and the clusters' visibility
+        runs, packed in the reference's order into the `al_*` tables, their used lengths into `al_sizes`. Returns the
+        number of kernel launches."""
+        assert "E" in self.stages, 'the annotation layout needs a batch built with stage "E"'
+        st = stream if stream is not None else torch.cuda.current_stream(self.device).cuda_stream
+        p = lambda t: t.data_ptr()
+        with torch.cuda.device(self.device):
+            _lib.call("s2d_annotation_layout", p(self.descs), self.nv, self.total_rows, p(self.vidinfo), p(self.rowinfo),
+                      p(self.winbits), p(self.rsbits), p(self.rebits), p(self.glabel), p(self.qframe), p(self.qlabel),
+                      p(self.grp_n), p(self.grp_one2x), p(self.area), p(self.gid_of), p(self.rle_bbox), p(self.str_off),
+                      p(self.rle_chars), self.str_cap, p(self.al_work), p(self.al_vann), p(self.al_ann), p(self.al_members),
+                      p(self.al_member_off), p(self.al_clusters), p(self.al_pairs), self.str_cap, p(self.al_chars),
+                      p(self.al_sizes), st)
+        return 3
+
+    def layout_views(self, sizes):
+        """Device views of the used part of every layout table, given a host copy of `al_sizes`."""
+        return {"vann": self.al_vann, **{k: getattr(self, "al_" + k)[:w * int(sizes[i])] for k, (w, i) in LAYOUT_TABLES.items()}}
+
     def annotations(self, results=None):
         """Stage E: per video the `annotations` list of the YTVIS json the reference writes for it
         (keymask_ident/annotations.py:8-140), or None when the video's final status is not 1 (the reference writes
-        none). Needs a batch built with "E" in its stages, after run() or replay(). `results`: this step's decode(),
-        when the caller has it already.
+        none). Needs a batch built with "E" in its stages, after run() or replay(). `results` is accepted for
+        compatibility and unused: the annotations no longer come from decode().
 
-        Built from decode()'s clusters, groupings and one2x and the device RLE tables, in the reference's order:
+        The device lays them out (layout(), after the stage-E capacities are settled) in the reference's order:
         cluster directories with candidates in lexicographic order of `cluster_{c}`, groups in lexicographic order
         of `group_{l}`, ids from 1 across the video. A group with two members on one frame keeps the member with the
-        largest label id (the reference keeps whichever PNG its directory listing returns last)."""
-        tab = self.rle_tables()
-        res = results if results is not None else self.decode(want_comps=False)
-        soff, chars, bbox = tab["str_off"], tab["chars"], tab["bbox"]
-        area = self.area.cpu().numpy().reshape(-1, S2D_MAX_LABELS)
-        gid_of = self.gid_of.cpu().numpy().reshape(-1, S2D_MAX_LABELS)
-        out = []
-        for vi, r in enumerate(res):
-            if r["status"] != 1:
-                out.append(None)
-                continue
-            d = self.host_descs[vi]
-            T, H, W, f0, r0 = d.T, d.H, d.W, d.frame0, d.row0
-            with_cands = [c for c, cl in enumerate(r["clusters"]) if any(x["candidates"] for x in cl["all_candidates"])]
-            groups_of = {gr["cluster_id"]: gr["overall_mask_ids_per_label"] for gr in r["groupings"]}
-            anns = []
-            for c in sorted(with_cands, key=lambda c: f"cluster_{c}"):
-                cname = f"cluster_{c}"
-                if cname not in r["one2x"]:
-                    continue
-                groups = groups_of.get(c, {})
-                for lab in sorted(groups, key=lambda l: f"group_{l}"):
-                    segs, boxes, areas = [None] * T, [None] * T, [None] * T
-                    for f, m in sorted(groups[lab], key=lambda fm: fm[1]):      # tie rule: the largest label id wins
-                        g = r0 + int(gid_of[f0 + f, m])
-                        segs[f] = {"size": [H, W], "counts": chars[soff[g]:soff[g + 1]]}
-                        x0, y0, x1, y1 = (int(v) for v in bbox[g])
-                        boxes[f] = [float(x0), float(y0), float(x1 - x0 + 1), float(y1 - y0 + 1)]
-                        areas[f] = int(area[f0 + f, m])
-                    anns.append({"video_id": 1, "iscrowd": 0, "height": H, "width": W, "length": T,
-                                 "segmentations": segs, "bboxes": boxes, "areas": areas, "category_id": 1,
-                                 "id": len(anns) + 1, "one2x": round(float(r["one2x"][cname][f"group_{lab}"]["avg_one2x"]), 2),
-                                 "visibility_ranges": [list(x) for x in r["clusters"][c]["ranges"]]})
-            out.append(anns)
-        return out
+        largest label id (the reference keeps whichever PNG its directory listing returns last). The host copies the
+        used part of the tables back and slices them into json objects."""
+        with torch.cuda.device(self.device):
+            self._settle_rle()
+            self.layout()
+            sizes = self.al_sizes.cpu().tolist()
+            tabs = {k: t.cpu().numpy() for k, t in self.layout_views(sizes).items()}
+            status = self.vidinfo.cpu().numpy()[3::S2D_VIDINFO_WORDS]
+        return annotations_from_layout(self.host_descs, status, tabs)
+
+
+# layout table -> (int32 / int64 / byte elements per entry, index of its entry count in al_sizes)
+LAYOUT_TABLES = {"ann": (7, 0), "members": (6, 1), "member_off": (1, 1), "chars": (1, 2), "clusters": (2, 3), "pairs": (2, 4)}
+
+
+def annotations_from_layout(descs, status, tabs):
+    """The `annotations` lists of a batch from host copies of its layout tables (Batch.layout_views): per video the
+    reference's json objects, None when `status` (vidinfo[3] per video) is not 1. Only slices: every choice was made
+    on the device."""
+    vann = tabs["vann"].reshape(-1, 2).tolist()
+    ann = tabs["ann"].reshape(-1, 7).tolist()
+    mem = tabs["members"].reshape(-1, 6).tolist()
+    moff = tabs["member_off"].tolist() + [len(tabs["chars"])]
+    chars = tabs["chars"].tobytes().decode("ascii")
+    clusters = tabs["clusters"].reshape(-1, 2).tolist()
+    pairs = tabs["pairs"].reshape(-1, 2).tolist()
+    out = []
+    for vi, d in enumerate(descs):
+        if int(status[vi]) != 1:
+            out.append(None)
+            continue
+        T, H, W = d.T, d.H, d.W
+        n, a0 = vann[vi]
+        anns = []
+        for k in range(n):
+            _, _, gn, gs, ci, m0, nm = ann[a0 + k]
+            segs, boxes, areas = [None] * T, [None] * T, [None] * T
+            for m in range(m0, m0 + nm):
+                f, x0, y0, x1, y1, a = mem[m]
+                segs[f] = {"size": [H, W], "counts": chars[moff[m]:moff[m + 1]]}
+                boxes[f] = [float(x0), float(y0), float(x1 - x0 + 1), float(y1 - y0 + 1)]
+                areas[f] = a
+            p0, npairs = clusters[ci]
+            anns.append({"video_id": 1, "iscrowd": 0, "height": H, "width": W, "length": T,
+                         "segmentations": segs, "bboxes": boxes, "areas": areas, "category_id": 1,
+                         "id": k + 1, "one2x": round(gs / gn, 2) if gn else 0.0,
+                         "visibility_ranges": [list(x) for x in pairs[p0:p0 + npairs]]})
+        out.append(anns)
+    return out
 
 
 def pack_vis_bits(vis: torch.Tensor) -> torch.Tensor:

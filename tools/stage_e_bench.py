@@ -8,7 +8,12 @@ Batch.annotations(), and - for comparison - the previous route on 4 of the video
 s2d_rle_encode, host string packing. A separate torch.profiler pass gives each kernel's time. The sha256 of the
 annotations of a direct run and of a CUDA-graph replay are both recorded (they must be equal).
 
-    python tools/stage_e_bench.py --out profiles/r03_stage_e_c2.json
+The annotation layout (s2d_annotation_layout, 3 kernels) is timed with CUDA events around Batch.layout(), and
+annotations() with a host clock (it ends in a device synchronise). HostPipeline's frames/s over the 64 videos (a pool
+of 8 distinct pinned videos cycled, chunks of 4, bit-packed flags: bench.py's e2e set-up) is measured with and without
+annotations, alternated in this one run.
+
+    python tools/stage_e_bench.py --out profiles/r04_annotation_layout_c2.json
 """
 from __future__ import annotations
 
@@ -43,7 +48,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_stage_e_c2.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r04_annotation_layout_c2.json"))
     args = ap.parse_args()
 
     import numpy as np
@@ -88,11 +93,24 @@ def main():
     t_lr, t_rs = ms(timers["label_rle"]), ms(timers["rle_strings"])
     med = lambda x: float(np.median(x))
 
-    # host side of stage E
+    # annotation layout on the device, then annotations() end to end (layout, copies, json objects)
+    bE.annotations()
+    lay = []
+    for _ in range(args.steps):
+        e0, e1 = ev(), ev()
+        e0.record()
+        bE.layout()
+        e1.record()
+        lay.append((e0, e1))
+    torch.cuda.synchronize()
+    t_lay = ms(lay)
+    hosts = []
+    for _ in range(3):
+        h0 = time.perf_counter()
+        anns = bE.annotations()
+        hosts.append(time.perf_counter() - h0)
+    t_host = min(hosts)
     res = bE.decode(want_comps=False)
-    h0 = time.perf_counter()
-    anns = bE.annotations(res)
-    t_host = time.perf_counter() - h0
     nkeymask = sum(sum(len(a["segmentations"]) - a["segmentations"].count(None) for a in x) for x in anns if x)
     sha_direct = sha(anns)
     bE.capture(p)
@@ -164,7 +182,11 @@ def main():
         "step_ms_without_E": {"median": med(t_0), "all": t_0},
         "keymask_rows": int(bE.total_rows), "annotated_keymasks": nkeymask, "counts": int(need[0]), "string_bytes": int(need[1]),
         "counts_capacity_first_guess_fit": bool(tab is not None and need[0] <= bE.rle_cap),
-        "annotations_host_s": t_host,
+        "annotations_host_s": t_host, "annotations_host_s_all": hosts,
+        "annotation_layout_ms": {"median": med(t_lay), "all": t_lay},
+        "annotation_layout_sizes": dict(zip(("annotations", "members", "string_bytes", "clusters", "range_pairs"),
+                                            bE.al_sizes.cpu().tolist())),
+        "hostpipe_frames_per_s": hostpipe_fps(vids, nv, T, dev, p, args.steps),
         "kernels_profiler_us": kern,
         "previous_route_4_videos": {"masks": n, "mask_plane_bytes": int(masks.numel()),
                                     "s2d_rle_encode_ms": med(ms(enc)), "host_pack_s": t_pack},
@@ -175,7 +197,35 @@ def main():
     with open(args.out, "w") as f:
         json.dump(out, f, indent=1)
     print(json.dumps({k: out[k] for k in ("card", "label_rle_ms", "rle_strings_ms", "label_rle_fraction_of_copy_peak",
-                                          "step_ms_with_E", "step_ms_without_E", "annotations_host_s")}, default=str)[:2000])
+                                          "step_ms_with_E", "step_ms_without_E", "annotations_host_s",
+                                          "annotation_layout_ms", "hostpipe_frames_per_s", "annotations_sha256_direct")},
+                     default=str)[:3000])
+
+
+def hostpipe_fps(vids, nv, T, dev, params, rounds):
+    """HostPipeline over the whole list with and without annotations, alternated (bench.py's e2e pool and chunks)"""
+    import torch
+
+    from s2d_b200.hostpipe import HostPipeline, HostVideo
+    from s2d_b200.pipeline import pack_vis_bits
+    chunk, npool = 4, 8
+    hv = [HostVideo(v.labels.cpu().pin_memory(), v.tracks.cpu().pin_memory(), pack_vis_bits(v.vis).cpu().pin_memory(),
+                    vis_bits=True, max_label=v.max_label) for v in vids[:npool]]
+    order = [hv[i % npool] for i in range(nv)]
+    pipes = {"without": HostPipeline(hv, dev, params, chunk=chunk),
+             "with_annotations": HostPipeline(hv, dev, params, chunk=chunk, annotations=True)}
+    for p in pipes.values():
+        p.run(order)                                   # warm-up: pinned host tables, buffer growth
+    t = {k: [] for k in pipes}
+    for _ in range(max(1, rounds // 3)):
+        for k, p in pipes.items():
+            torch.cuda.synchronize(dev)
+            t0 = time.perf_counter()
+            p.run(order)
+            t[k].append(nv * T / (time.perf_counter() - t0))
+    out = {k: {"median": float(sorted(v)[len(v) // 2]), "all": v} for k, v in t.items()}
+    out["reruns_with_annotations"] = pipes["with_annotations"].reruns
+    return out
 
 
 if __name__ == "__main__":
