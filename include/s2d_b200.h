@@ -281,6 +281,33 @@ int s2d_annotation_layout(const s2d_video_desc* descs, int nvideos, int64_t tota
                           int32_t* ann, int32_t* members, int64_t* member_off, int32_t* clusters, int32_t* pairs,
                           int64_t capacity, char* chars, int64_t* sizes, void* stream);
 
+/* The annotation json of stage E: for every video whose vidinfo[3] (final status) is 1, the exact text of its YTVIS
+ * `annotations` list - the bytes of Python's json.dumps of the list annotations_from_layout (s2d_b200/pipeline.py)
+ * builds from the same tables: default separators ", " and ": ", keys in the order video_id, iscrowd, height, width,
+ * length, segmentations, bboxes, areas, category_id, id, one2x, visibility_ranges; null for a frame without a member;
+ * segmentations {"size": [H, W], "counts": "..."}; boxes [x0.0, y0.0, w.0, h.0] as Python prints float(int); areas
+ * and range pairs as ints; "[]" for a video without annotation. Two rules decide byte equality:
+ *   - '\' (92), the only character of the RLE alphabet chr(48)..chr(111) that json escapes, is written as "\\";
+ *   - one2x = repr(round(gs / gn, 2)) (0.0 when gn == 0): x = gs / gn is one IEEE double division, k = 100 x rounded
+ *     half to even from x's exact binary value (1/8 -> 0.12, 3/8 -> 0.38, 1/200 -> 0.01), printed as k / 100 with
+ *     trailing zeros stripped and at least one decimal. For |gs|, |gn| < 2^31 that is Python's shortest repr.
+ * Inputs: the outputs of s2d_annotation_layout as they sit on the device (vann, ann, members, member_off, chars,
+ * clusters, pairs, and sizes, whose counts are read on the device), T / H / W of the descriptors, vidinfo[3]. nchars is
+ * the capacity the layout was given for `chars`: strings are read only below it. When stage E's string capacity was
+ * short the layout's sizes[2] exceeds it and the text is incomplete (the caller re-runs stage E, the layout and this
+ * call). nvideos <= 65535.
+ * Output: video v's text at out + video_off[v] .. out + video_off[v + 1] (int64 [nvideos + 1]); videos whose status is
+ * not 1 get an empty range. *needed = video_off[nvideos], the bytes the batch needs; nothing is written at or past
+ * `capacity` (the caller re-runs this call alone with a larger buffer: its inputs are intact). Two passes with a scan
+ * between them, no host round trip: the call can be captured in a CUDA graph together with the layout.
+ * work: int32 scratch of s2d_annotation_json_work_ints(total_rows, nvideos) elements, 8-byte aligned. */
+int s2d_annotation_json_work_ints(int64_t total_rows, int nvideos, int64_t* out);
+int s2d_annotation_json(const s2d_video_desc* descs, int nvideos, int64_t total_rows, const int32_t* vidinfo,
+                        const int32_t* vann, const int32_t* ann, const int32_t* members, const int64_t* member_off,
+                        const char* chars, int64_t nchars, const int32_t* clusters, const int32_t* pairs,
+                        const int64_t* sizes,
+                        int32_t* work, int64_t capacity, char* out, int64_t* video_off, int64_t* needed, void* stream);
+
 /* K4a. Scores and selection per candidate query: iou = hits/uniq (double), match bit when
  * iou > matching_threshold (cotracker_matching.py:710), one-to-many flag when >= one2x_frames
  * frames hold more than one mask with iou > one2x_iou (cotracker_matching.py:1082-1111).

@@ -64,6 +64,8 @@ SIGNATURES = {
     "s2d_rle_strings": [_P, _P, _I, _L, _P, _L, _P, _P, _P, _P],
     "s2d_annotation_layout_work_ints": [_L, _I, C.POINTER(C.c_int64)],
     "s2d_annotation_layout": [_P, _I, _L] + [_P] * 15 + [_L, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P],
+    "s2d_annotation_json_work_ints": [_L, _I, C.POINTER(C.c_int64)],
+    "s2d_annotation_json": [_P, _I, _L] + [_P] * 6 + [_L] + [_P] * 4 + [_L, _P, _P, _P, _P],
     "s2d_select": [_P, _I, _I, _L, _P, _P, _P, _P, _D, _D, _I, _P, _P, _P, _P, _P],
     "s2d_group_work_ints": [_L, _I, C.POINTER(C.c_int64)],
     "s2d_group": [_P, _I, _I, _I, _L, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P],

@@ -10,7 +10,7 @@ against 14 ms of kernels), which is why the wire format matters: visibility flag
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Union
 
 import torch
 
@@ -44,16 +44,24 @@ class HostPipeline:
     video's YTVIS annotation list as well. Before a staging set is reused, the host reads the stage-E needs and layout
     sizes of the chunk it holds (the next chunk's copies are in flight meanwhile): a short capacity is grown and stage
     E and the layout re-run on that set, whose label maps are still staged; then only the used part of the layout
-    tables is copied back."""
+    tables is copied back.
+
+    `annotations="json"` adds the annotation json (Batch.serialize) after the layout instead: the json text of every
+    video's annotation list is made on the device, and only its used bytes and the video offsets are copied back, with
+    no Python annotation objects built. The host reads the stage-E needs and the json size before a set is reused;
+    a short stage-E capacity re-runs stage E, the layout and the json, a short json buffer the json call alone."""
 
     RESULT_TABLES = ("vidinfo", "clusterinfo", "rowinfo", "glabel", "one2x")
 
     def __init__(self, like: Sequence[HostVideo], device, params: Params = Params(), chunk: Optional[int] = None,
-                 annotations: bool = False):
+                 annotations: Union[bool, str] = False):
+        if annotations not in (False, True, "json"):
+            raise ValueError(f"annotations must be False, True or 'json', not {annotations!r}")
         self.device = torch.device(device)
         self.params = params
         self.chunk = int(chunk) if chunk else len(like)
-        self.annotations = bool(annotations)
+        self.annotations = annotations if annotations == "json" else bool(annotations)
+        self.json = annotations == "json"
         assert len(like) in (self.chunk, 2 * self.chunk)
         halves = [list(like[:self.chunk]), list(like[-self.chunk:])]
         self.sigs = [[v.signature() for v in h] for h in halves]
@@ -70,7 +78,9 @@ class HostPipeline:
             self.compute_stream = torch.cuda.Stream(self.device)
         self.host_results: List[dict] = []          # one set of pinned result tables per chunk, grown on first use
         self.host_sizes: List[torch.Tensor] = []    # annotations: per chunk stage E's need (2) and the layout sizes (5)
-        self.host_layout: List[dict] = []           # annotations: per chunk pinned layout tables, grown on demand
+        #                                             or, with "json", the json bytes (1)
+        self.host_layout: List[dict] = []           # annotations: per chunk pinned layout tables (with "json": the json
+        #                                             text and video offsets), grown on demand
         self.h2d_bytes = 0
         self.d2h_bytes = 0
         self.launches = 0
@@ -80,7 +90,8 @@ class HostPipeline:
         """All videos, chunk by chunk. Returns one dict of pinned host result tables per chunk (owned by the pipeline,
         overwritten by the next run); with annotations=True each dict also holds "annotations": per video of the chunk,
         in list order, its annotation list (keymask_ident.annotations.write_video_annotations) or None when its status
-        is not 1. Synchronises the device once at the end, and with annotations twice per chunk as well."""
+        is not 1; with annotations="json" it holds "annotation_json" instead: per video the json text of that list as
+        bytes, or None. Synchronises the device once at the end, and with annotations twice per chunk as well."""
         assert len(videos) % self.chunk == 0, "the list must be a whole number of chunks"
         nchunks = len(videos) // self.chunk
         while len(self.host_results) < nchunks:      # first call only: pinned result tables for every chunk
@@ -88,7 +99,7 @@ class HostPipeline:
             self.host_results.append({k: torch.empty(getattr(b0, k).shape, dtype=getattr(b0, k).dtype, pin_memory=True)
                                       for k in self.RESULT_TABLES})
             if self.annotations:
-                self.host_sizes.append(torch.empty(7, dtype=torch.int64, pin_memory=True))
+                self.host_sizes.append(torch.empty(3 if self.json else 7, dtype=torch.int64, pin_memory=True))
                 self.host_layout.append({})
         done = [None, None]
         self.h2d_bytes = self.d2h_bytes = self.launches = self.reruns = 0
@@ -116,6 +127,8 @@ class HostPipeline:
                     self.launches += b.run(self.params)
                     if self.annotations:
                         self.launches += b.layout()
+                        if self.json:
+                            self.launches += b.serialize()
                         self._copy_sizes(c, b)
                     for k in self.RESULT_TABLES:
                         hbuf = self.host_results[c][k]
@@ -137,6 +150,13 @@ class HostPipeline:
     def _assemble(self, c):
         """chunk c's annotation lists from its pinned layout tables (copied back already)"""
         b = self.sets[c % 2][1]
+        if self.json:
+            hl = self.host_layout[c]
+            off = hl["video_off"].tolist()
+            text = hl["text"][:off[-1]].numpy().tobytes()
+            self.host_results[c]["annotation_json"] = [text[off[v]:off[v + 1]] if off[v + 1] > off[v] else None
+                                                       for v in range(b.nv)]
+            return
         hs = self.host_sizes[c].tolist()
         n = {k: w * int(hs[2 + i]) for k, (w, i) in LAYOUT_TABLES.items()}
         n["vann"] = 2 * b.nv
@@ -147,7 +167,7 @@ class HostPipeline:
     def _copy_sizes(self, c, b):
         hs = self.host_sizes[c]
         hs[:2].copy_(b.rle_need, non_blocking=True)
-        hs[2:].copy_(b.al_sizes, non_blocking=True)
+        hs[2:].copy_(b.aj_need if self.json else b.al_sizes, non_blocking=True)
         self.d2h_bytes += hs.numel() * hs.element_size()
 
     def _collect(self, c, done):
@@ -158,6 +178,8 @@ class HostPipeline:
         st = self.copy_streams[c % 2]
         done.synchronize()
         hs = self.host_sizes[c]
+        if self.json:
+            return self._collect_json(c, b, st)
         with torch.cuda.stream(st):
             while not b.rle_fits(hs[:2].tolist()):
                 b.grow_rle(hs[:2].tolist())
@@ -171,6 +193,37 @@ class HostPipeline:
                     hl[k] = torch.empty(t.numel() + t.numel() // 4 + 64, dtype=t.dtype, pin_memory=True)
                 hl[k][:t.numel()].copy_(t, non_blocking=True)
                 self.d2h_bytes += t.numel() * t.element_size()
+            copied = torch.cuda.Event()
+            copied.record()
+        return copied
+
+    def _collect_json(self, c, b, st):
+        """_collect for annotations="json": re-run what a short capacity left incomplete (stage E, the layout and the json
+        when a stage-E buffer was short, the json call alone when its text buffer was), then copy the used json bytes
+        and the video offsets to pinned host buffers."""
+        hs = self.host_sizes[c]
+        with torch.cuda.stream(st):
+            while True:
+                need = hs.tolist()
+                if not b.rle_fits(need[:2]):
+                    b.grow_rle(need[:2])
+                    self.launches += b.run(self.params, stages="E") + b.layout() + b.serialize()
+                elif need[2] > b.aj_cap:
+                    b.grow_json(need[2])
+                    self.launches += b.serialize()
+                else:
+                    break
+                self.reruns += 1
+                self._copy_sizes(c, b)
+                st.synchronize()
+            hl = self.host_layout[c]
+            n = int(hs[2])
+            if "text" not in hl or hl["text"].numel() < n:
+                hl["text"] = torch.empty(n + n // 4 + 64, dtype=torch.uint8, pin_memory=True)
+                hl["video_off"] = torch.empty(b.nv + 1, dtype=torch.int64, pin_memory=True)
+            hl["text"][:n].copy_(b.aj_out[:n], non_blocking=True)
+            hl["video_off"].copy_(b.aj_video_off, non_blocking=True)
+            self.d2h_bytes += n + hl["video_off"].numel() * 8
             copied = torch.cuda.Event()
             copied.record()
         return copied

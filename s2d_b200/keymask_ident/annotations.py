@@ -174,19 +174,30 @@ def _video_entry(video_path):
             "file_names": [os.path.join(video_name, f) for f in video_files], "flickr_url": "", "id": 1}
 
 
+_CATEGORIES = [{"supercategory": "object", "id": 1, "name": "fg"}]
+
+
 def _dump_video_json(video, annotations, annotation_output_path, video_path):
     """`{videos, annotations, categories}` of one video to <annotation_output_path>/<video name>.json
-    (annotations.py:131-140)."""
+    (annotations.py:131-140). `annotations` is the list, or its json text as bytes (Batch.annotation_json): then the
+    other parts are json.dumps'ed around it, which gives the file json.dump writes for the list."""
     os.makedirs(annotation_output_path, exist_ok=True)
-    with open(os.path.join(annotation_output_path, f"{os.path.basename(video_path)}.json"), "w") as f:
-        json.dump({"videos": [video], "annotations": annotations,
-                   "categories": [{"supercategory": "object", "id": 1, "name": "fg"}]}, f)
+    path = os.path.join(annotation_output_path, f"{os.path.basename(video_path)}.json")
+    if isinstance(annotations, (bytes, bytearray)):
+        with open(path, "wb") as f:
+            f.write(b'{"videos": ' + json.dumps([video]).encode() + b', "annotations": ' + bytes(annotations) +
+                    b', "categories": ' + json.dumps(_CATEGORIES).encode() + b"}")
+        return
+    with open(path, "w") as f:
+        json.dump({"videos": [video], "annotations": annotations, "categories": _CATEGORIES}, f)
 
 
 def write_video_annotations(video_path, annotations, annotation_output_path):
     """The json write_annotation_for_video produces, for annotations computed elsewhere - the device stage E of the
-    batched path (s2d_b200.pipeline: Batch.annotations, discover_keymasks(..., annotations=True)). Nothing is written
-    for a video without annotations (None: the reference writes no json for a failed video) or without images."""
+    batched path (s2d_b200.pipeline: Batch.annotations, discover_keymasks(..., annotations=True)). `annotations` may
+    also be the json text of the list as bytes (Batch.annotation_json, discover_keymasks(..., annotations="json")):
+    the file is the same. Nothing is written for a video without annotations (None: the reference writes no json for
+    a failed video) or without images."""
     if annotations is None:
         return
     video = _video_entry(video_path)

@@ -12,7 +12,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 from dataclasses import dataclass, field
-from typing import List, Optional
+from typing import List, Optional, Union
 
 import numpy as np
 import torch
@@ -204,6 +204,8 @@ class Batch:
         # stage E: COCO RLE of every keymask row from the label maps (counts, offsets, boxes) and its strings
         self.rle_work = self.rle_counts = self.rle_off = self.rle_bbox = self.rle_need = None
         self.str_work = self.str_off = self.rle_chars = self.al_work = self.al_chars = None
+        self.aj_work = self.aj_out = None
+        self.aj_cap = 0
         self.rle_cap = self.str_cap = 0
         if "E" in st:
             assert "L" in st and "D" in st, 'stage "E" reads K0\'s gid_of ("L") and the final status of K4 ("D")'
@@ -230,6 +232,14 @@ class Batch:
             # first guess: blob-like maps have about two edges per (object, column); too small re-runs (annotations())
             cap = sum(descs[i].T * 8 * descs[i].W for i in range(nv)) + 2 * row0
             self._alloc_rle(cap, 3 * cap)
+            # annotation json (s2d_annotation_json): the text buffer is allocated by the first serialize(), sized as the
+            # layout's string capacity plus 128 bytes of fixed text per row (segmentation header, box, area, separators,
+            # nulls); a short guess re-runs the json call alone
+            _lib.call("s2d_annotation_json_work_ints", row0, nv, C.byref(n))
+            self.aj_work = z(n.value)
+            self.aj_video_off = torch.zeros(nv + 1, dtype=torch.int64, device=dev)
+            self.aj_need = torch.zeros(1, dtype=torch.int64, device=dev)
+            self.aj_out, self.aj_cap = None, self.str_cap + 128 * row0
         self._graph = None
         self.kernel_launches_per_run = 0
         # persistent TMA-fed votes kernel (the library falls back by itself when P is odd)
@@ -572,6 +582,47 @@ class Batch:
             status = self.vidinfo.cpu().numpy()[3::S2D_VIDINFO_WORDS]
         return annotations_from_layout(self.host_descs, status, tabs)
 
+    def serialize(self, stream=None) -> int:
+        """Enqueue the annotation json (s2d_annotation_json) of the layout tables on `stream` (default: torch's current
+        stream): per video the text of its `annotations` list at aj_out[aj_video_off[v]:aj_video_off[v + 1]], the bytes
+        the batch needs in `aj_need`. Follows layout(). The first call allocates the text buffer, so call it once
+        before capturing it in a graph. Returns the number of kernel launches."""
+        assert "E" in self.stages, 'the annotation json needs a batch built with stage "E"'
+        if self.aj_out is None:
+            self.grow_json(self.aj_cap)
+        st = stream if stream is not None else torch.cuda.current_stream(self.device).cuda_stream
+        p = lambda t: t.data_ptr()
+        with torch.cuda.device(self.device):
+            _lib.call("s2d_annotation_json", p(self.descs), self.nv, self.total_rows, p(self.vidinfo), p(self.al_vann),
+                      p(self.al_ann), p(self.al_members), p(self.al_member_off), p(self.al_chars), self.str_cap,
+                      p(self.al_clusters), p(self.al_pairs), p(self.al_sizes), p(self.aj_work), self.aj_cap, p(self.aj_out),
+                      p(self.aj_video_off), p(self.aj_need), st)
+        return 3
+
+    def grow_json(self, need: int):
+        """(Re)allocate the json text buffer for at least `need` bytes; serialize() has to be run again."""
+        self.aj_cap = max(int(need), self.aj_cap if self.aj_out is not None else 0)
+        self.aj_out = torch.empty(max(1, self.aj_cap), dtype=torch.uint8, device=self.device)
+
+    def annotation_json(self):
+        """Per video the json text of its `annotations` list as bytes, byte-identical to
+        `json.dumps(self.annotations()[v]).encode()`, or None when the video's final status is not 1. Needs a batch
+        built with "E" in its stages, after run() or replay(). The stage-E capacities are settled as in annotations(),
+        then the layout and the json are enqueued on the device; only the used bytes and the offsets are copied back.
+        When the text buffer was short it is grown and the json call alone re-run (the layout tables are intact).
+        keymask_ident.annotations.write_video_annotations writes the bytes into the video's file."""
+        with torch.cuda.device(self.device):
+            self._settle_rle()
+            self.layout()
+            self.serialize()
+            need = int(self.aj_need.item())
+            if need > self.aj_cap:
+                self.grow_json(need)
+                self.serialize()
+            off = self.aj_video_off.cpu().tolist()
+            text = self.aj_out[:need].cpu().numpy().tobytes()
+        return [text[off[v]:off[v + 1]] if off[v + 1] > off[v] else None for v in range(self.nv)]
+
 
 # layout table -> (int32 / int64 / byte elements per entry, index of its entry count in al_sizes)
 LAYOUT_TABLES = {"ann": (7, 0), "members": (6, 1), "member_off": (1, 1), "chars": (1, 2), "clusters": (2, 3), "pairs": (2, 4)}
@@ -640,16 +691,22 @@ def _setbits(words: np.ndarray, limit: int):
 
 
 def discover_keymasks(videos: List[VideoInput], params: Params = Params(), want_comps: bool = True,
-                      annotations: bool = False):
+                      annotations: Union[bool, str] = False):
     """Public in-memory entry point: run stages A-D for a batch of videos on their device and
     return one result dict per video. annotations=True runs stage E as well: each dict gains "annotations", the
     YTVIS annotation list the reference writes for the video (None when its status is not 1; see
-    Batch.annotations and keymask_ident.annotations.write_video_annotations)."""
+    Batch.annotations and keymask_ident.annotations.write_video_annotations). annotations="json" gains
+    "annotation_json" instead: the json text of that list as bytes, serialised on the device (Batch.annotation_json)."""
+    if annotations not in (False, True, "json"):
+        raise ValueError(f"annotations must be False, True or 'json', not {annotations!r}")
     b = Batch(videos, stages="LVBDE" if annotations else "LVBD")
     b.run(params)
     torch.cuda.synchronize(b.device)
     res = b.decode(want_comps=want_comps)
-    if annotations:
+    if annotations == "json":
+        for r, a in zip(res, b.annotation_json()):
+            r["annotation_json"] = a
+    elif annotations:
         for r, a in zip(res, b.annotations(res)):
             r["annotations"] = a
     return res

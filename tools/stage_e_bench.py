@@ -202,8 +202,9 @@ def main():
                      default=str)[:3000])
 
 
-def hostpipe_fps(vids, nv, T, dev, params, rounds):
-    """HostPipeline over the whole list with and without annotations, alternated (bench.py's e2e pool and chunks)"""
+def hostpipe_fps(vids, nv, T, dev, params, rounds, modes=(("without", False), ("with_annotations", True))):
+    """HostPipeline over the whole list for each (name, annotations=) of `modes`, alternated (bench.py's e2e pool and
+    chunks); by default without and with annotations"""
     import torch
 
     from s2d_b200.hostpipe import HostPipeline, HostVideo
@@ -212,8 +213,7 @@ def hostpipe_fps(vids, nv, T, dev, params, rounds):
     hv = [HostVideo(v.labels.cpu().pin_memory(), v.tracks.cpu().pin_memory(), pack_vis_bits(v.vis).cpu().pin_memory(),
                     vis_bits=True, max_label=v.max_label) for v in vids[:npool]]
     order = [hv[i % npool] for i in range(nv)]
-    pipes = {"without": HostPipeline(hv, dev, params, chunk=chunk),
-             "with_annotations": HostPipeline(hv, dev, params, chunk=chunk, annotations=True)}
+    pipes = {k: HostPipeline(hv, dev, params, chunk=chunk, annotations=a) for k, a in modes}
     for p in pipes.values():
         p.run(order)                                   # warm-up: pinned host tables, buffer growth
     t = {k: [] for k in pipes}
@@ -224,7 +224,10 @@ def hostpipe_fps(vids, nv, T, dev, params, rounds):
             p.run(order)
             t[k].append(nv * T / (time.perf_counter() - t0))
     out = {k: {"median": float(sorted(v)[len(v) // 2]), "all": v} for k, v in t.items()}
-    out["reruns_with_annotations"] = pipes["with_annotations"].reruns
+    if "with_annotations" in pipes:
+        out["reruns_with_annotations"] = pipes["with_annotations"].reruns
+    out["reruns"] = {k: p.reruns for k, p in pipes.items()}
+    out["d2h_bytes"] = {k: p.d2h_bytes for k, p in pipes.items()}
     return out
 
 
