@@ -247,6 +247,38 @@ int s2d_label_rle(const s2d_video_desc* descs, int nvideos, int max_T, int max_H
 int s2d_rle_strings(const int32_t* counts, const int64_t* offsets, int N, int64_t ncounts, int32_t* work,
                     int64_t capacity, char* chars, int64_t* str_offsets, int64_t* needed, void* stream);
 
+/* The inverse of s2d_rle_strings: run-length lists of N COCO compressed-RLE strings on the device (maskApi.c rleFrString,
+ * which every consumer of the annotations calls through mask_util.decode before it has a mask; annotations.py:94-106 and
+ * convert_results_to_annotations.py:70-81 produce and read these strings). chars: the strings back to back, string n at
+ * chars[str_offsets[n] .. str_offsets[n + 1]) (str_offsets int64 [N + 1], on the device). A value ends at a character
+ * whose bit 0x20 is clear (c = byte - 48, for every byte as maskApi computes it); its 5-bit groups are sign-extended from
+ * bit 0x10 of the last; count m > 2 is the value plus count m - 2.
+ *   counts         int32, the lists back to back, list n at counts[count_offsets[n] .. count_offsets[n + 1])
+ *   count_offsets  int64 [N + 1];  *needed = count_offsets[N], the total number of counts (at most the number of
+ *                  characters). Nothing is written at or past `capacity` (re-run with a larger buffer when *needed >
+ *                  capacity)
+ *   status         int32 [N]: 0, or 1 for a malformed string: its last character still has the continuation bit set (the
+ *                  unfinished value is dropped), or a count falls outside [0, 2^31). Other strings are not affected.
+ * No host round trip: the call can be captured in a CUDA graph. work: int32 scratch of
+ * s2d_rle_from_strings_work_ints(N, nchars) elements. */
+int s2d_rle_from_strings_work_ints(int N, int64_t nchars, int64_t* out);
+int s2d_rle_from_strings(const char* chars, const int64_t* str_offsets, int N, int32_t* work, int64_t capacity,
+                         int32_t* counts, int64_t* count_offsets, int32_t* status, int64_t* needed, void* stream);
+
+/* Binary masks of N run-length lists (maskApi.c rleDecode, what mask_util.decode returns per segmentation), each on its
+ * own: counts / count_offsets [N + 1] as s2d_rle_from_strings writes them (counts are read as unsigned, as maskApi does),
+ * heights / widths int32 [N], out_offsets int64 [N] (all on the device). Mask n is written to
+ * out + out_offsets[n] as H * W bytes, row-major, value 0 or 1 (runs are column-major, the first a run of zeros); the
+ * offsets may leave gaps (frames of an [A, T, H, W] tensor without a segmentation), which are not touched. Sizes may
+ * differ within one call; H, W <= 65535 and H * W < 2^31. status int32 [N] is OR-ed with 2 when the runs do not sum to
+ * H * W (or the size is out of range, then nothing is written for that mask): pixels past the sum are 0 and runs past
+ * H * W are ignored. No byte outside a mask's own H * W bytes is written. No host round trip: the call can be captured
+ * in a CUDA graph. work: int32 scratch of s2d_rle_decode_work_ints(N, count_offsets[N]) elements, 8-byte aligned. */
+int s2d_rle_decode_work_ints(int N, int64_t ncounts, int64_t* out);
+int s2d_rle_decode(const int32_t* counts, const int64_t* count_offsets, int N, const int32_t* heights,
+                   const int32_t* widths, const int64_t* out_offsets, int32_t* work, uint8_t* out, int32_t* status,
+                   void* stream);
+
 /* Annotation layout of stage E: which keymask rows become which YTVIS annotation, in the reference's order
  * (annotations.py:8-140 walks `cluster_*` and `group_*` directories sorted as strings), as compact tables. Reads the
  * tables of stages L, B, D and E already on the device; only videos whose vidinfo[3] (final status) is 1 get entries.

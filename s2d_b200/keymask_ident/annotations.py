@@ -4,6 +4,8 @@
 in one batch on the GPU (s2d_rle_encode: column-major run lengths, area, bounding box; s2d_rle_strings: the
 base-48 string packing of maskApi.c rleToString). Batched callers that got their annotations from
 s2d_b200.pipeline (stage E on the device) write the same json with write_video_annotations.
+coco_rle.decode_batch and decode_video_annotations turn the strings back into masks on the device (mask_util.decode:
+s2d_rle_from_strings, s2d_rle_decode).
 pycocotools is not installable in the build container, so parity at the RLE boundary is pinned by
 the published algorithm and by decode round trips only (tests/test_dropin_gpu.py)."""
 from __future__ import annotations
@@ -131,6 +133,123 @@ class coco_rle:
         so = soff.cpu().numpy()
         return [text[so[i]:so[i + 1]] for i in range(n)]
 
+    @staticmethod
+    def counts_from_strings_device(strings):
+        """rleFrString of N strings (str or bytes, ASCII) on the device, in one launch sequence (s2d_rle_from_strings) ->
+        (counts int32, offsets int64 [N + 1], status int32 [N]), device tensors: list n is counts[offsets[n]:offsets[n +
+        1]], status[n] = 1 marks a malformed string (its last character continues, or a count falls outside [0, 2^31)).
+        No host synchronisation."""
+        dev = _engine.device()
+        blobs = [s.encode("ascii") if isinstance(s, str) else bytes(s) for s in strings]
+        counts = torch.empty(max(1, sum(len(b) for b in blobs)), dtype=torch.int32, device=dev)
+        status = torch.empty(len(blobs), dtype=torch.int32, device=dev)
+        if not blobs:
+            return counts[:0], torch.zeros(1, dtype=torch.int64, device=dev), status
+        return counts, coco_rle._parse_device(blobs, dev, counts, status), status
+
+    @staticmethod
+    def _parse_device(blobs, dev, counts, status):
+        """s2d_rle_from_strings of the byte strings `blobs` into counts (capacity: one count per character at most, so
+        it is never short) and status [len(blobs)]; returns the device offsets [len(blobs) + 1]."""
+        from s2d_b200 import _lib
+        n = len(blobs)
+        offs = np.zeros(n + 1, np.int64)
+        offs[1:] = np.cumsum([len(b) for b in blobs])
+        nchars = int(offs[-1])
+        assert counts.numel() >= nchars and status.numel() >= n
+        chars = torch.frombuffer(bytearray(b"".join(blobs) or b"\0"), dtype=torch.uint8).to(dev)
+        d_off = torch.from_numpy(offs).to(dev)
+        need = C.c_int64()
+        _lib.call("s2d_rle_from_strings_work_ints", n, nchars, C.byref(need))
+        work = torch.empty(need.value, dtype=torch.int32, device=dev)
+        count_off = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        needed = torch.empty(1, dtype=torch.int64, device=dev)
+        _lib.call("s2d_rle_from_strings", chars.data_ptr(), d_off.data_ptr(), n, work.data_ptr(), counts.numel(),
+                  counts.data_ptr(), count_off.data_ptr(), status.data_ptr(), needed.data_ptr(),
+                  torch.cuda.current_stream(dev).cuda_stream)
+        return count_off
+
+    @staticmethod
+    def _decode_into(rles, out, out_offsets):
+        """rleDecode of the RLE dicts `rles` into the uint8 device buffer `out`, mask i at byte out_offsets[i] (host
+        int64): one parse launch sequence for all compressed strings, one decode launch sequence for all masks. Returns
+        the device status int32 [len(rles)] (1: malformed string, 2: runs do not sum to H * W). Uncompressed counts
+        (lists) and non-ASCII strings (host from_string) are range-checked here and uploaded as they are."""
+        from s2d_b200 import _lib
+        dev = out.device
+        n = len(rles)
+        blobs, s_idx, lists, l_idx = [], [], [], []
+        for i, r in enumerate(rles):
+            c = r["counts"]
+            if isinstance(c, str):
+                try:
+                    c = c.encode("ascii")
+                except UnicodeEncodeError:
+                    try:
+                        c = coco_rle.from_string(c)
+                    except IndexError:
+                        raise ValueError(f"segmentation {i}: malformed RLE string") from None
+            if isinstance(c, (bytes, bytearray)):
+                blobs.append(c)
+                s_idx.append(i)
+                continue
+            c = np.asarray(c, dtype=np.int64).reshape(-1)
+            if c.size and (c.min() < 0 or c.max() >= 2 ** 31):
+                raise ValueError(f"segmentation {i}: RLE counts outside [0, 2^31)")
+            lists.append(c.astype(np.int32))
+            l_idx.append(i)
+        # lists first, then the parsed strings: one contiguous counts buffer and one offsets array for the decode
+        l_off = np.zeros(len(lists) + 1, np.int64)
+        l_off[1:] = np.cumsum([len(x) for x in lists])
+        nl = int(l_off[-1])
+        nchars = sum(len(b) for b in blobs)
+        counts = torch.empty(nl + max(1, nchars), dtype=torch.int32, device=dev)
+        if nl:
+            counts[:nl] = torch.from_numpy(np.concatenate(lists)).to(dev)
+        status = torch.zeros(n, dtype=torch.int32, device=dev)
+        count_off = torch.from_numpy(l_off).to(dev)
+        if blobs:
+            s_off = coco_rle._parse_device(blobs, dev, counts[nl:], status[len(lists):])
+            count_off = torch.cat([count_off[:-1], s_off + nl])
+        order = l_idx + s_idx
+        size = np.asarray([[int(rles[i]["size"][0]), int(rles[i]["size"][1])] for i in order], np.int32).reshape(-1, 2)
+        hs = torch.from_numpy(np.ascontiguousarray(size[:, 0])).to(dev)
+        ws = torch.from_numpy(np.ascontiguousarray(size[:, 1])).to(dev)
+        oo = torch.from_numpy(np.asarray(out_offsets, np.int64)[order]).to(dev)
+        need = C.c_int64()
+        _lib.call("s2d_rle_decode_work_ints", n, nl + nchars, C.byref(need))
+        work = torch.empty(need.value, dtype=torch.int32, device=dev)
+        _lib.call("s2d_rle_decode", counts.data_ptr(), count_off.data_ptr(), n, hs.data_ptr(), ws.data_ptr(), oo.data_ptr(),
+                  work.data_ptr(), out.data_ptr(), status.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        back = torch.empty_like(status)
+        back[torch.tensor(order, dtype=torch.int64, device=dev)] = status
+        return back
+
+    @staticmethod
+    def decode_batch(rles, check=True):
+        """mask_util.decode on the device: one RLE dict ({"size": [h, w], "counts": str | bytes | list}) -> uint8 [H, W];
+        a list of them, all of one size (ValueError otherwise) -> uint8 [N, H, W]. Unlike pycocotools, which returns
+        [H, W, N], the mask index comes first. Values are 0 / 1. With check=True a malformed string or runs that do not
+        sum to H * W raise ValueError naming the first such index; with check=False the call returns (masks, status) -
+        status int32 ([N] or a scalar; 1: malformed string, 2: wrong sum) - without synchronising the host."""
+        single = isinstance(rles, dict)
+        lst = [rles] if single else list(rles)
+        sizes = {(int(r["size"][0]), int(r["size"][1])) for r in lst}
+        if len(sizes) > 1:
+            raise ValueError(f"decode_batch: masks of different sizes {sorted(sizes)} in one call")
+        h, w = sizes.pop() if sizes else (0, 0)
+        dev = _engine.device()
+        buf = torch.empty(max(1, len(lst) * h * w), dtype=torch.uint8, device=dev)
+        out = buf[:len(lst) * h * w].view(len(lst), h, w)
+        status = (coco_rle._decode_into(lst, buf, np.arange(len(lst), dtype=np.int64) * h * w) if lst
+                  else torch.zeros(0, dtype=torch.int32, device=dev))
+        if single:
+            out, status = out[0], status[0]
+        if not check:
+            return out, status
+        _raise_on_status(status.reshape(-1), "segmentation")
+        return out
+
 
 def rle_area_bbox_batch(rles):
     """[(area int, bbox [x, y, w, h] floats)] of COCO RLE dicts ({"size": [h, w], "counts": str | bytes | list})
@@ -203,6 +322,57 @@ def write_video_annotations(video_path, annotations, annotation_output_path):
     video = _video_entry(video_path)
     if video is not None:
         _dump_video_json(video, annotations, annotation_output_path, video_path)
+
+
+def _raise_on_status(status, what):
+    bad = torch.nonzero(status).reshape(-1).cpu()
+    if bad.numel():
+        i = int(bad[0])
+        s = int(status[i])
+        why = "malformed RLE string" if s & 1 else "runs do not sum to H * W"
+        raise ValueError(f"{what} {i}: {why} (status {s}; {bad.numel()} bad in all)")
+
+
+def decode_video_annotations(annotations, check=True):
+    """The masks of one video's YTVIS `annotations` - the list Batch.annotations() returns, its json text as bytes
+    (Batch.annotation_json()) or the "annotations" of a loaded file - as uint8 [A, T, H, W] on the device: annotation a,
+    frame t is mask_util.decode of segmentations[t], zero where the segmentation is null. All segmentations go through
+    one parse and one decode launch sequence. check=True raises ValueError on a malformed segmentation (named by
+    annotation and frame); check=False returns (masks, status int32 [A, T]) without synchronising the host."""
+    if isinstance(annotations, (bytes, bytearray, str)):
+        annotations = json.loads(annotations)
+    dev = _engine.device()
+    A = len(annotations)
+    T = len(annotations[0]["segmentations"]) if A else 0
+    rles, slots, hw = [], [], set()
+    for a, ann in enumerate(annotations):
+        segs = ann["segmentations"]
+        if len(segs) != T:
+            raise ValueError(f"annotation {a}: {len(segs)} frames, annotation 0 has {T}")
+        for t, s in enumerate(segs):
+            if s is not None:
+                rles.append(s)
+                slots.append(a * T + t)
+                hw.add((int(s["size"][0]), int(s["size"][1])))
+    if len(hw) > 1:
+        raise ValueError(f"decode_video_annotations: segmentations of different sizes {sorted(hw)}")
+    H, W = hw.pop() if hw else ((int(annotations[0]["height"]), int(annotations[0]["width"])) if A else (0, 0))
+    buf = torch.zeros(max(1, A * T * H * W), dtype=torch.uint8, device=dev)
+    out = buf[:A * T * H * W].view(A, T, H, W)
+    status = torch.zeros(A * T, dtype=torch.int32, device=dev)
+    if rles:
+        status[torch.tensor(slots, dtype=torch.int64, device=dev)] = coco_rle._decode_into(
+            rles, buf, np.asarray(slots, np.int64) * H * W)
+    status = status.view(A, T)
+    if not check:
+        return out, status
+    bad = torch.nonzero(status).cpu()
+    if bad.shape[0]:
+        a, t = (int(x) for x in bad[0])
+        s = int(status[a, t])
+        why = "malformed RLE string" if s & 1 else "runs do not sum to H * W"
+        raise ValueError(f"annotation {a} frame {t}: {why} (status {s}; {bad.shape[0]} bad in all)")
+    return out
 
 
 def write_annotation_for_video(video_path, cluster_masks_path, annotation_output_path, visibility_data):
