@@ -296,16 +296,7 @@ class Batch:
             call("select", 1, "s2d_select", d, nv, self.max_Nm, self.total_mw, p(self.hits), p(self.uniq),
                  p(self.gid_of), p(self.rowinfo), params.matching_threshold, params.one2x_iou,
                  params.one2x_frames, p(self.mbits), p(self.one2x), p(self.nmatch), p(self.vidinfo), st)
-            if self.gram is not None:
-                for i, off in self._gram_videos:           # match rows -> u8 planes -> G = X X^T (tcgen05 kind::i8)
-                    hd = self.host_descs[i]
-                    mb = self.mbits.data_ptr() + 4 * hd.mbits_off
-                    call("group", 1, "s2d_unpack_bits", mb, hd.Nm, hd.NW, hd.NW * 32, p(self.gram_planes), st)
-                    call("group", 2, "s2d_overlap_i8", p(self.gram_planes), hd.Nm, p(self.gram_planes), hd.Nm, hd.NW * 32,
-                         self.gram.data_ptr() + 4 * off, st)
-            call("group", 8, "s2d_group_gram", d, nv, self.max_Nm, self.max_NW, self.total_rows, p(self.mbits),
-                 p(self.rowinfo), p(self.one2x), p(self.grpwork), p(self.glabel), p(self.grp_n),
-                 p(self.grp_one2x), p(self.vidinfo), p(self.clusterinfo), p(self.gram), p(self.gram_off), st)
+            self._enqueue_group(call, st, True)
         if "E" in stages:
             call("label_rle", 5, "s2d_label_rle", d, nv, self.max_T, self.max_H, self.max_W, self.max_Nm,
                  self.total_frames, self.total_rows, p(self.gid_of), p(self.vidinfo), p(self.rle_work), self.rle_cap,
@@ -314,6 +305,31 @@ class Batch:
                  p(self.str_work), self.str_cap, p(self.rle_chars), p(self.str_off), p(self.rle_need) + 8, st)
         self.kernel_launches_per_run = launches
         return launches
+
+    def _enqueue_group(self, call, st, gram: bool):
+        """DBSCAN #2 and the grouping of stage D on the match tables in place (mbits, rowinfo, one2x, vidinfo). Videos with a
+        Gram buffer first contract their match rows with themselves; `gram=False` takes every video's distances from the
+        bit rows instead."""
+        p = lambda t: t.data_ptr() if t is not None else None
+        use = gram and self.gram is not None
+        if use:
+            for i, off in self._gram_videos:               # match rows -> u8 planes -> G = X X^T (tcgen05 kind::i8)
+                hd = self.host_descs[i]
+                mb = self.mbits.data_ptr() + 4 * hd.mbits_off
+                call("group", 1, "s2d_unpack_bits", mb, hd.Nm, hd.NW, hd.NW * 32, p(self.gram_planes), st)
+                call("group", 2, "s2d_overlap_i8", p(self.gram_planes), hd.Nm, p(self.gram_planes), hd.Nm, hd.NW * 32,
+                     self.gram.data_ptr() + 4 * off, st)
+        call("group", 8, "s2d_group_gram", p(self.descs), self.nv, self.max_Nm, self.max_NW, self.total_rows, p(self.mbits),
+             p(self.rowinfo), p(self.one2x), p(self.grpwork), p(self.glabel), p(self.grp_n), p(self.grp_one2x),
+             p(self.vidinfo), p(self.clusterinfo), p(self.gram) if use else None, p(self.gram_off) if use else None, st)
+
+    def group(self, stream=None, gram: bool = True):
+        """Enqueue stage D's grouping alone (what run() does after s2d_select) on the match tables as they stand: callers
+        that fill mbits / rowinfo / one2x / vidinfo themselves, and re-runs of one step's grouping with `gram=False`."""
+        assert "D" in self.stages, 'the grouping needs a batch built with stage "D"'
+        st = stream if stream is not None else torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            self._enqueue_group(lambda tag, nk, name, *args: _lib.call(name, *args), st, gram)
 
     def _alloc_rle(self, counts_cap: int, chars_cap: int):
         self.rle_cap, self.str_cap = int(counts_cap), int(chars_cap)
