@@ -279,6 +279,44 @@ int s2d_rle_decode(const int32_t* counts, const int64_t* count_offsets, int N, c
                    const int32_t* widths, const int64_t* out_offsets, int32_t* work, uint8_t* out, int32_t* status,
                    void* stream);
 
+/* PNG label maps (the colour-coded mask frames every video starts from) decoded to packed RGB on the device: what
+ * cv2.imread(path, IMREAD_COLOR) returns in load_masks / load_image_robust (crw_utils.py:310-346, 714-767,
+ * cotracker_occlusions.py:22-85, cotracker_matching.py:22-84), in RGB order, for non-interlaced files. The host parses
+ * the chunks; this call inflates each file's zlib stream (a warp per file: stored, fixed- and dynamic-Huffman blocks),
+ * undoes the row filters and converts each row: palette lookup, gray replicated to R = G = B (1/2/4-bit gray scaled to
+ * 0-255), 1/2/4-bit samples unpacked, 16-bit samples reduced to their high byte, alpha and tRNS dropped.
+ *   zdata       the files' IDAT payloads joined, file n at zdata[z_offsets[n] .. z_offsets[n + 1]) (z_offsets int64
+ *               [N + 1]), the 2-byte zlib header and the adler32 trailer included
+ *   descs       s2d_png_desc [N] (on the device, 8-byte aligned): the IHDR fields, the palette, and where the file's
+ *               filtered scanlines (H * (1 + rowbytes) bytes, in the work area) and its RGB frame (H * W * 3 bytes,
+ *               row-major, at rgb_out + rgb_offset) go. Ranges of different files must not overlap; sizes may differ.
+ *   status      int32 [N], written for every file: 0, or an OR of the S2D_PNG_BAD_* bits. A flagged file's RGB range
+ *               holds no defined pixels; other files are not affected. No byte outside a file's own ranges is written.
+ * No host round trip: the call can be captured in a CUDA graph. work: int32 scratch of
+ * s2d_png_decode_work_ints(N, raw_bytes) elements, 16-byte aligned, where raw_bytes covers every file's
+ * raw_offset + H * (1 + rowbytes). */
+#define S2D_PNG_MAX_ROWBYTES 16384            /* wider rows (and frames above S2D_PNG_MAX_RAW_BYTES) get S2D_PNG_BAD_DESC */
+#define S2D_PNG_MAX_RAW_BYTES (1 << 30)
+#define S2D_PNG_BAD_DEFLATE 1                 /* zlib header, block type, code, symbol 286/287, distance 30/31 or one
+                                                 reaching before the stream's start or past its window; data short of
+                                                 the final block or left after the adler32 */
+#define S2D_PNG_BAD_SIZE 2                    /* the stream ends short of, or would run past, H * (1 + rowbytes) bytes */
+#define S2D_PNG_BAD_FILTER 4                  /* a filter byte greater than 4 */
+#define S2D_PNG_BAD_ADLER 8                   /* adler32 mismatch */
+#define S2D_PNG_BAD_DESC 16                   /* (colour type, bit depth) pair, size or palette size out of range */
+#define S2D_PNG_BAD_INDEX 32                  /* a palette index at or past the palette's entries */
+typedef struct s2d_png_desc {
+    int32_t width, height, bit_depth, color_type;   /* IHDR; colour type 0, 2, 3, 4 or 6 */
+    int64_t raw_offset;                             /* byte offset of the filtered scanlines in the work area */
+    int64_t rgb_offset;                             /* byte offset of the RGB frame in rgb_out */
+    int32_t palette_size;                           /* PLTE entries (colour type 3), 1-256 */
+    int32_t reserved;
+    uint8_t palette[768];                           /* PLTE, RGB */
+} s2d_png_desc;                                     /* 808 bytes */
+int s2d_png_decode_work_ints(int N, int64_t raw_bytes, int64_t* out);
+int s2d_png_decode(const uint8_t* zdata, const int64_t* z_offsets, const s2d_png_desc* descs, int N, int32_t* work,
+                   uint8_t* rgb_out, int32_t* status, void* stream);
+
 /* Annotation layout of stage E: which keymask rows become which YTVIS annotation, in the reference's order
  * (annotations.py:8-140 walks `cluster_*` and `group_*` directories sorted as strings), as compact tables. Reads the
  * tables of stages L, B, D and E already on the device; only videos whose vidinfo[3] (final status) is 1 get entries.

@@ -66,6 +66,8 @@ SIGNATURES = {
     "s2d_rle_from_strings": [_P, _P, _I, _P, _L, _P, _P, _P, _P, _P],
     "s2d_rle_decode_work_ints": [_I, _L, C.POINTER(C.c_int64)],
     "s2d_rle_decode": [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P],
+    "s2d_png_decode_work_ints": [_I, _L, C.POINTER(C.c_int64)],
+    "s2d_png_decode": [_P, _P, _P, _I, _P, _P, _P, _P],
     "s2d_annotation_layout_work_ints": [_L, _I, C.POINTER(C.c_int64)],
     "s2d_annotation_layout": [_P, _I, _L] + [_P] * 15 + [_L, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P],
     "s2d_annotation_json_work_ints": [_L, _I, C.POINTER(C.c_int64)],

@@ -135,13 +135,18 @@ def visibility_windows(V: np.ndarray, qframe, qlabel, visibility_threshold: floa
 
 
 def color_frames_to_labels(rgb_frames: np.ndarray):
-    """f1 on the GPU: [F,H,W,3] uint8 RGB frames -> ([F,H,W] uint8 label ids on the device, colours per
-    frame). Same ids as crw_utils.rgb_to_label_ids (rank of the RGB tuple among the non-black colours)."""
+    """f1 on the GPU: [F,H,W,3] uint8 RGB frames (numpy, or a tensor already on the device) -> ([F,H,W] uint8 label
+    ids on the device, colours per frame). Same ids as crw_utils.rgb_to_label_ids (rank of the RGB tuple among the
+    non-black colours)."""
     import ctypes as C
     from s2d_b200 import _lib
     F, H, W, _ = rgb_frames.shape
-    dev = device()
-    rgb = torch.from_numpy(np.ascontiguousarray(rgb_frames)).to(dev)
+    if torch.is_tensor(rgb_frames):
+        rgb = rgb_frames.contiguous()
+        dev = rgb.device
+    else:
+        dev = device()
+        rgb = torch.from_numpy(np.ascontiguousarray(rgb_frames)).to(dev)
     n = C.c_int64()
     _lib.call("s2d_color_to_labels_work_ints", F, C.byref(n))
     work = torch.empty(n.value, dtype=torch.int32, device=dev)

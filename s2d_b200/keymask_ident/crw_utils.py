@@ -118,6 +118,17 @@ def load_masks(mask_folder: str):
     paths = sorted(glob.glob(os.path.join(mask_folder, "*.png")))
     if not paths:
         raise ValueError(f"No .png masks found in {mask_folder!r}")
+    if torch.cuda.is_available():
+        # PNG decode and colour -> id on the GPU (s2d_png_decode, s2d_color_to_labels); files the device decoder does
+        # not take go through load_image_robust, as below
+        from s2d_b200 import png
+        frames = png.load_rgb_frames(paths)
+        if not frames:
+            raise RuntimeError("No valid mask images could be read.")
+        if len({tuple(f.shape) for f in frames}) == 1:
+            return png.rgb_frames_to_labels(frames).cpu().to(torch.int64)[..., None]
+        frames = [f.cpu().numpy() for f in frames]
+        return torch.from_numpy(np.stack([rgb_to_label_ids(f)[..., None] for f in frames], axis=0))
     frames = []
     for p in paths:
         bgr = load_image_robust(p)
@@ -126,14 +137,6 @@ def load_masks(mask_folder: str):
         frames.append(cv2.cvtColor(bgr, cv2.COLOR_BGR2RGB))
     if not frames:
         raise RuntimeError("No valid mask images could be read.")
-    if torch.cuda.is_available() and len({f.shape for f in frames}) == 1:
-        # colour -> id on the GPU (s2d_color_to_labels); the host only decodes the PNGs
-        try:
-            from . import _engine
-        except ImportError:
-            import _engine
-        labels, _ = _engine.color_frames_to_labels(np.stack(frames, axis=0))
-        return labels.cpu().to(torch.int64)[..., None]
     return torch.from_numpy(np.stack([rgb_to_label_ids(f)[..., None] for f in frames], axis=0))
 
 
