@@ -255,27 +255,15 @@ aj_scan_kernel(int nvideos, int64_t total_rows, const int32_t* __restrict__ vidi
                const int64_t* __restrict__ sizes, int64_t* __restrict__ alen, int64_t* __restrict__ video_off,
                int64_t* __restrict__ needed, int64_t capacity, char* __restrict__ out) {
     __shared__ int64_t wsum[AJ_SCAN_THREADS / 32];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     const int64_t A = sizes[0];
     S2D_DEV_ASSERT(A >= 0 && A <= total_rows);
-    auto scan = [&](int64_t x, int64_t& total) {                           // exclusive block prefix, total = block sum
-        int64_t incl = x;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int64_t u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int64_t before = 0;
-        total = 0;
-        for (int w = 0; w < AJ_SCAN_THREADS / 32; ++w) { const int64_t s = wsum[w]; if (w < warp) before += s; total += s; }
-        __syncthreads();
-        return before + incl - x;
-    };
     int64_t carry = 0;
     for (int64_t base = 0; base < A; base += AJ_SCAN_THREADS) {
         const int64_t i = base + tid;
         const int64_t x = i < A ? alen[i] : 0;
         int64_t tot;
-        const int64_t ex = scan(x, tot);
+        const int64_t ex = block_excl_scan<AJ_SCAN_THREADS>(x, wsum, tot);
         if (i < A) alen[i] = carry + ex;
         carry += tot;
     }
@@ -293,7 +281,7 @@ aj_scan_kernel(int nvideos, int64_t total_rows, const int32_t* __restrict__ vidi
             len = empty ? 2 : alen[a0 + n] - alen[a0];
         }
         int64_t tot;
-        const int64_t ex = carry + scan(len, tot);
+        const int64_t ex = carry + block_excl_scan<AJ_SCAN_THREADS>(len, wsum, tot);
         if (v < nvideos) {
             video_off[v] = ex;
             if (empty) {

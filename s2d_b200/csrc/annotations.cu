@@ -39,22 +39,6 @@ __device__ __forceinline__ uint64_t al_key(int rank, int group, int frame, int l
 __device__ __forceinline__ bool al_same_group(uint64_t a, uint64_t b) { return (a >> 18) == (b >> 18); }
 __device__ __forceinline__ bool al_same_frame(uint64_t a, uint64_t b) { return (a >> 8) == (b >> 8); }
 
-// exclusive prefix of x over the block (every thread calls it); *total = block sum. wsum: AL_THREADS / 32 slots.
-template <typename T>
-__device__ T al_block_scan(T x, T* wsum, T& total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    T incl = x;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const T u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
-    if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
-    T before = 0;
-    total = 0;
-    for (int w = 0; w < AL_THREADS / 32; ++w) { const T s = wsum[w]; if (w < warp) before += s; total += s; }
-    __syncthreads();
-    return before + incl - x;
-}
-
 // set bits below T of a cluster's run-start (run-end) row
 __device__ __forceinline__ uint32_t al_word(const uint32_t* row, int w, int T) {
     const int valid = T - 32 * w;
@@ -190,7 +174,7 @@ al_scan_kernel(int nvideos, const int64_t* __restrict__ vcnt, int64_t* __restric
             const int v = base + threadIdx.x;
             const int64_t x = v < nvideos ? vcnt[(int64_t)v * AL_VWORDS + q] : 0;
             int64_t tot;
-            const int64_t ex = al_block_scan(x, wsum, tot);
+            const int64_t ex = block_excl_scan<AL_THREADS>(x, wsum, tot);
             if (v < nvideos) {
                 vfirst[(int64_t)v * AL_NCOUNT + q] = carry + ex;
                 if (q == 0) { vann[2 * v] = (int32_t)x; vann[2 * v + 1] = (int32_t)(carry + ex); }
@@ -260,9 +244,9 @@ al_write_kernel(const s2d_video_desc* __restrict__ descs, const int32_t* __restr
         const int64_t src = in ? str_off[r] : 0;
         const int len = mem ? (int)(str_off[r + 1] - src) : 0;
         int64_t tot_a, tot_m, tot_c;
-        const int64_t ea = al_block_scan<int64_t>(gs, wsum, tot_a);
-        const int64_t em = al_block_scan<int64_t>(mem, wsum, tot_m);
-        const int64_t ec = al_block_scan<int64_t>(len, wsum, tot_c);
+        const int64_t ea = block_excl_scan<AL_THREADS, int64_t>(gs, wsum, tot_a);
+        const int64_t em = block_excl_scan<AL_THREADS, int64_t>(mem, wsum, tot_m);
+        const int64_t ec = block_excl_scan<AL_THREADS, int64_t>(len, wsum, tot_c);
         const int64_t mi = M0 + mem_carry + em, dst = C0 + chr_carry + ec;
         if (gs) {
             const int rank = (int)(key >> 56), c = cl[rank], l = glabel[r];

@@ -85,6 +85,37 @@ __device__ __forceinline__ int4 ld_stream(const int4* p) {
 
 __device__ __forceinline__ int warp_sum(int v) { return __reduce_add_sync(0xffffffffu, v); }
 
+// inclusive sum of x over the 32 lanes of a full warp (1-D blocks: lane = threadIdx.x & 31)
+template <typename T>
+__device__ __forceinline__ T warp_incl_scan(T x) {
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const T u = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += u; }
+    return x;
+}
+
+// exclusive prefix of x over a block of THREADS threads (every thread calls it); total = the block sum. wsum: THREADS / 32
+// shared slots. Ends with a barrier, so the caller may reuse wsum at once. The warp sums are read eight at a time: a full
+// unroll keeps all 32 of a 1024-thread block in flight, which costs up to 64 registers per thread.
+template <int THREADS, typename T>
+__device__ __forceinline__ T block_excl_scan(T x, T* wsum, T& total) {
+    S2D_DEV_ASSERT(blockDim.x == THREADS);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const T incl = warp_incl_scan(x);
+    if (lane == 31) wsum[warp] = incl;
+    __syncthreads();
+    T before = 0;
+    total = 0;
+#pragma unroll 8
+    for (int w = 0; w < THREADS / 32; ++w) { const T s = wsum[w]; if (w < warp) before += s; total += s; }
+    __syncthreads();
+    return before + incl - x;
+}
+
+// out[0, n] = exclusive prefix of in[0, n) as int64 (out[n] = the sum), *total = the sum: one 1024-thread CTA on st.
+// Returns 0, or -2 with the error set when the launch fails. Defined in label_rle.cu.
+int launch_offsets(const int32_t* in, int64_t n, int64_t* out, int64_t* total, cudaStream_t st);
+
 __device__ __forceinline__ int cdiv(int a, int b) { return (a + b - 1) / b; }
 
 }  // namespace s2d

@@ -52,29 +52,17 @@ __device__ __forceinline__ void csa(uint32_t& carry, uint32_t& sum, uint32_t a, 
 // instead of launching - and immediately retiring - a CTA per (problem, block) slot (round 1: 23 k CTAs per pass on the
 // C2 batch, 2 944 of them with work).
 __global__ void __launch_bounds__(1024) db_worklist_kernel(const DbProblem* __restrict__ problems, int n, int32_t* __restrict__ wl) {
-    __shared__ int ws0[32], ws1[32];
-    __shared__ int run0, run1;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) { run0 = 0; run1 = 0; }
-    __syncthreads();
+    __shared__ int wsum[32];
+    const int tid = threadIdx.x;
+    int run0 = 0, run1 = 0;
     for (int base = 0; base < n; base += 1024) {
         const int i = base + tid;
         const int nb = i < n ? (problems[i].N + DB_ROWS_I - 1) / DB_ROWS_I : 0;
-        const int np = nb * (nb + 1) / 2;
-        int x0 = nb, x1 = np;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int y0 = __shfl_up_sync(0xffffffffu, x0, o), y1 = __shfl_up_sync(0xffffffffu, x1, o);
-            if (lane >= o) { x0 += y0; x1 += y1; }
-        }
-        if (lane == 31) { ws0[warp] = x0; ws1[warp] = x1; }
-        __syncthreads();
-        int b0 = run0, b1 = run1, t0 = 0, t1 = 0;
-        for (int w = 0; w < 32; ++w) { if (w < warp) { b0 += ws0[w]; b1 += ws1[w]; } t0 += ws0[w]; t1 += ws1[w]; }
-        if (i < n) { wl[i] = b0 + x0 - nb; wl[n + 1 + i] = b1 + x1 - np; }
-        __syncthreads();
-        if (tid == 0) { run0 += t0; run1 += t1; }
-        __syncthreads();
+        int t0, t1;
+        const int e0 = block_excl_scan<1024>(nb, wsum, t0);
+        const int e1 = block_excl_scan<1024>(nb * (nb + 1) / 2, wsum, t1);
+        if (i < n) { wl[i] = run0 + e0; wl[n + 1 + i] = run1 + e1; }
+        run0 += t0; run1 += t1;
     }
     if (tid == 0) { wl[n] = run0; wl[2 * n + 1] = run1; }
 }

@@ -12,7 +12,7 @@
 //
 //   pass 1  lr_strip_kernel<false>   edges per (frame, strip, label) of every keymask row
 //   scan    lr_frame_scan_kernel     per frame and label: exclusive prefix over strips; runs per row = edges + 1
-//           lr_scan_kernel           runs per row -> int64 offsets of the rows in one flat `counts` buffer
+//           offsets_kernel           runs per row -> int64 offsets of the rows in one flat `counts` buffer
 //   pass 2  lr_strip_kernel<true>    edge positions written in order at offsets[row] + strip prefix + rank
 //   diff    lr_diff_kernel           a warp per row turns its edges into run lengths in place, bounding box
 // Each frame's bytes are read from HBM twice (pass 1 and pass 2). Nothing is written at or past `capacity`.
@@ -192,31 +192,30 @@ lr_frame_scan_kernel(const s2d_video_desc* __restrict__ descs, const int32_t* __
     rowruns[d.row0 + g] = run + 1;
 }
 
-// out[0] = 0, out[i + 1] = in[0] + ... + in[i] (int64), *total = out[n]. One CTA.
-constexpr int LR_SCAN_THREADS = 1024;
-__global__ void __launch_bounds__(LR_SCAN_THREADS)
-lr_scan_kernel(const int32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out, int64_t* __restrict__ total) {
-    __shared__ int64_t wsum[LR_SCAN_THREADS / 32];
-    __shared__ int64_t running;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) { running = 0; out[0] = 0; }
-    __syncthreads();
-    for (int64_t base = 0; base < n; base += LR_SCAN_THREADS) {
-        const int64_t i = base + tid;
-        const int64_t x = i < n ? (int64_t)in[i] : 0;
-        int64_t incl = x;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int64_t u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int64_t before = running, tot = 0;
-        for (int w = 0; w < LR_SCAN_THREADS / 32; ++w) { const int64_t s = wsum[w]; if (w < warp) before += s; tot += s; }
-        if (i < n) out[i + 1] = before + incl;
-        __syncthreads();
-        if (tid == 0) running += tot;
-        __syncthreads();
+// out[i] = in[0] + ... + in[i - 1] (int64) for i = 0 .. n, *total = out[n]. One CTA; the next step's inputs are
+// loaded before the current step's scan, so the load latency overlaps the scan's barriers instead of adding to them.
+constexpr int OFFSETS_THREADS = 1024;
+__global__ void __launch_bounds__(OFFSETS_THREADS)
+offsets_kernel(const int32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out, int64_t* __restrict__ total) {
+    __shared__ int64_t wsum[OFFSETS_THREADS / 32];
+    int64_t carry = 0;
+    int x = threadIdx.x < n ? in[threadIdx.x] : 0;
+    for (int64_t base = 0; base < n; base += OFFSETS_THREADS) {
+        const int64_t i = base + threadIdx.x, next = i + OFFSETS_THREADS;
+        const int xn = next < n ? in[next] : 0;
+        int64_t tot;
+        const int64_t ex = block_excl_scan<OFFSETS_THREADS, int64_t>(x, wsum, tot);
+        if (i < n) out[i] = carry + ex;
+        carry += tot;
+        x = xn;
     }
-    if (tid == 0) *total = running;
+    if (threadIdx.x == 0) { out[n] = carry; *total = carry; }
+}
+
+int launch_offsets(const int32_t* in, int64_t n, int64_t* out, int64_t* total, cudaStream_t st) {
+    offsets_kernel<<<1, OFFSETS_THREADS, 0, st>>>(in, n, out, total);
+    S2D_CHECK_LAUNCH("offsets_kernel");
+    return 0;
 }
 
 // A warp per keymask row: its edges e_0 < ... < e_{n-1} (column-major positions) become the run lengths
@@ -303,9 +302,7 @@ rs_kernel(const int32_t* __restrict__ counts, const int64_t* __restrict__ offset
         int x = i < nc ? rs_value(c, i) : 0;
         const int len = i < nc ? rs_len(x) : 0;
         if (WRITE) {
-            int incl = len;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
+            const int incl = warp_incl_scan(len);
             int64_t p = pos + incl - len;
             for (int k = 0; k < len; ++k, ++p) {
                 int ch = x & 0x1F;
@@ -367,8 +364,7 @@ extern "C" int s2d_label_rle(const s2d_video_desc* descs, int nvideos, int max_T
     S2D_CHECK_LAUNCH("lr_strip_kernel<count>");
     lr_frame_scan_kernel<<<dim3(max_T, nvideos), S2D_MAX_LABELS, 0, st>>>(descs, vidinfo, gid_of, max_strips, scnt, rowruns);
     S2D_CHECK_LAUNCH("lr_frame_scan_kernel");
-    lr_scan_kernel<<<1, LR_SCAN_THREADS, 0, st>>>(rowruns, total_rows, offsets, needed);
-    S2D_CHECK_LAUNCH("lr_scan_kernel");
+    if (const int rc = launch_offsets(rowruns, total_rows, offsets, needed, st)) return rc;
     lr_strip_kernel<true><<<grid, nw * 32, smem, st>>>(descs, vidinfo, gid_of, stage, max_strips, scnt, offsets,
                                                               capacity, counts);
     S2D_CHECK_LAUNCH("lr_strip_kernel<write>");
@@ -387,8 +383,7 @@ extern "C" int s2d_rle_strings(const int32_t* counts, const int64_t* offsets, in
     const int blocks = (N + RS_WARPS - 1) / RS_WARPS;
     rs_kernel<false><<<blocks, RS_WARPS * 32, 0, st>>>(counts, offsets, N, ncounts, work, nullptr, capacity, chars);
     S2D_CHECK_LAUNCH("rs_kernel<length>");
-    lr_scan_kernel<<<1, LR_SCAN_THREADS, 0, st>>>(work, N, str_offsets, needed);
-    S2D_CHECK_LAUNCH("lr_scan_kernel");
+    if (const int rc = launch_offsets(work, N, str_offsets, needed, st)) return rc;
     rs_kernel<true><<<blocks, RS_WARPS * 32, 0, st>>>(counts, offsets, N, ncounts, work, str_offsets, capacity, chars);
     S2D_CHECK_LAUNCH("rs_kernel<write>");
     return 0;

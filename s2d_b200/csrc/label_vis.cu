@@ -119,7 +119,7 @@ frame_tables_kernel(const s2d_video_desc* __restrict__ descs, const int32_t* __r
                     int32_t* __restrict__ vidinfo) {
     const s2d_video_desc d = descs[blockIdx.x];
     __shared__ int first[FT_MAX_T + 1];
-    __shared__ int wsum[8];
+    __shared__ int wsum[S2D_MAX_LABELS / 32];
     const int tid = threadIdx.x, w = tid >> 5, lane = tid & 31;
     const int T = min(d.T, FT_MAX_T);
     // pass 1: objects per frame (present labels minus the smallest one)
@@ -136,15 +136,8 @@ frame_tables_kernel(const s2d_video_desc* __restrict__ descs, const int32_t* __r
     int v[4], s = 0;
 #pragma unroll
     for (int k = 0; k < 4; ++k) { const int t = tid * 4 + k; v[k] = t < T ? first[t] : 0; s += v[k]; }
-    int x = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-    if (lane == 31) wsum[w] = x;
-    __syncthreads();
-    int before = 0, total_obj = 0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { const int t = wsum[k]; if (k < w) before += t; total_obj += t; }
-    int run = before + x - s;
+    int total_obj;
+    int run = block_excl_scan<S2D_MAX_LABELS>(s, wsum, total_obj);
 #pragma unroll
     for (int k = 0; k < 4; ++k) { const int t = tid * 4 + k; if (t < T) first[t] = run; run += v[k]; }
     __syncthreads();

@@ -133,9 +133,7 @@ __device__ bool build_table(InflateSmem& s, const uint8_t* lens, int n, uint32_t
     for (int base = 0; base < (1 << root); base += 32) {
         const int p = base + lane;
         const int b = s.sub[p];
-        int sz = b ? 1 << b : 0, incl = sz;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
+        const int sz = b ? 1 << b : 0, incl = warp_incl_scan(sz);
         if (b) { S2D_DEV_ASSERT(p < (1 << root)); tab[p] = (uint32_t)(off + incl - sz) | ((uint32_t)b << 16) | PI_PTR; }
         off += __shfl_sync(0xffffffffu, incl, 31);
     }

@@ -80,15 +80,13 @@ __global__ void __launch_bounds__(RLE_THREADS)
 rle_runs_kernel(const uint32_t* __restrict__ colbits, int H, int W, int HW, int max_runs,
                 int32_t* __restrict__ edges, int32_t* __restrict__ counts, int32_t* __restrict__ nruns) {
     __shared__ int wsum[RLE_THREADS / 32];
-    __shared__ int running;
-    const int n = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int n = blockIdx.x, tid = threadIdx.x;
     const uint32_t* cb = colbits + (int64_t)n * W * HW;
     int32_t* ed = edges + (int64_t)n * max_runs;
     int32_t* ct = counts + (int64_t)n * max_runs;
     const int nwords = W * HW;
     const uint32_t tailmask = (H & 31) ? ((1u << (H & 31)) - 1u) : 0xFFFFFFFFu;   // valid rows of a column's last word
-    if (tid == 0) running = 0;
-    __syncthreads();
+    int running = 0;
     for (int base = 0; base < nwords; base += RLE_THREADS) {
         const int i = base + tid;
         uint32_t t = 0;
@@ -104,16 +102,8 @@ rle_runs_kernel(const uint32_t* __restrict__ colbits, int H, int W, int HW, int 
             }
             t = (b ^ ((b << 1) | prev)) & (j == HW - 1 ? tailmask : 0xFFFFFFFFu);
         }
-        // block-wide exclusive scan of popc(t)
-        const int c = __popc(t);
-        int incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int before = running, total = 0;
-        for (int w = 0; w < RLE_THREADS / 32; ++w) { const int s = wsum[w]; if (w < warp) before += s; total += s; }
-        int idx = before + incl - c;
+        int total;
+        int idx = running + block_excl_scan<RLE_THREADS>(__popc(t), wsum, total);
         while (t) {                                   // edges: column-major position of every transition
             const int bit = __ffs(t) - 1;
             t &= t - 1;
@@ -121,9 +111,7 @@ rle_runs_kernel(const uint32_t* __restrict__ colbits, int H, int W, int HW, int 
             if (idx < max_runs) ed[idx] = x * H + j * 32 + bit;
             ++idx;
         }
-        __syncthreads();
-        if (tid == 0) running += total;
-        __syncthreads();
+        running += total;
     }
     // run k = edges[k] - edges[k-1] (edges[-1] = 0), the last run ends at H * W. A mask that starts with a
     // set pixel has a transition at position 0, i.e. a leading zero-length run, exactly like rleEncode.
@@ -198,10 +186,7 @@ rle_area_bbox_kernel(const int32_t* __restrict__ counts, const int64_t* __restri
         const int j = base + lane;
         S2D_DEV_ASSERT(j >= m || j < nr);
         const unsigned v = j < m ? (unsigned)c[j] : 0u;
-        unsigned incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const unsigned u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
-        const unsigned cc = carry + incl;
+        const unsigned cc = carry + warp_incl_scan(v);
         const unsigned t = cc - (unsigned)(j & 1);
         const unsigned y = t % h, x = (t - y) / h;
         // x of the preceding even boundary: the previous lane's (or the previous chunk's last even one)

@@ -2,7 +2,7 @@
 //
 //   s2d_rle_from_strings (maskApi.c rleFrString for N strings back to back)
 //     rp_count_kernel     warp per string: number of values = characters whose continuation bit 0x20 is clear
-//     rp_scan_kernel      one CTA: exclusive prefix -> count_offsets [N + 1], needed
+//     offsets_kernel      one CTA (launch_offsets): exclusive prefix -> count_offsets [N + 1], needed
 //     rp_write_kernel     warp per string, 32 characters per step: a ballot of the value ends, a segmented OR scan
 //                         assembles each value from its 5-bit groups, and two plain warp scans run the parity chains
 //   s2d_rle_decode (maskApi.c rleDecode, each mask independently)
@@ -27,7 +27,6 @@
 namespace s2d {
 
 constexpr int RP_WARPS = 8;                    // strings per CTA
-constexpr int RP_SCAN_THREADS = 1024;
 constexpr int RD_SCAN_WARPS = 8;               // masks per CTA of the run-start scan
 constexpr int RD_TC = 128;                     // tile columns = threads of rd_tile_kernel
 constexpr int RD_TR = 64;                      // tile rows
@@ -52,35 +51,6 @@ rp_count_kernel(const char* __restrict__ chars, const int64_t* __restrict__ str_
     }
     cnt = __reduce_add_sync(0xffffffffu, cnt);
     if (lane == 0) nvals[n] = cnt;
-}
-
-// in [n] int32 -> out [n + 1] int64 exclusive prefix (out[n] = total), *total
-__global__ void __launch_bounds__(RP_SCAN_THREADS)
-rp_scan_kernel(const int32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out, int64_t* __restrict__ total) {
-    __shared__ int64_t wsum[RP_SCAN_THREADS / 32];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    int64_t carry = 0;
-    for (int64_t base = 0; base < n; base += RP_SCAN_THREADS) {
-        const int64_t i = base + tid;
-        const int64_t x = i < n ? (int64_t)in[i] : 0;
-        int64_t incl = x;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int64_t u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int64_t before = 0, tot = 0;
-        for (int w = 0; w < RP_SCAN_THREADS / 32; ++w) { const int64_t s = wsum[w]; if (w < warp) before += s; tot += s; }
-        if (i < n) out[i] = carry + before + incl - x;
-        carry += tot;
-        __syncthreads();
-    }
-    if (tid == 0) { out[n] = carry; *total = carry; }
-}
-
-__device__ __forceinline__ uint32_t warp_scan_u32(uint32_t x, int lane) {
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const uint32_t u = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += u; }
-    return x;
 }
 
 __global__ void __launch_bounds__(RP_WARPS * 32)
@@ -127,8 +97,8 @@ rp_write_kernel(const char* __restrict__ chars, const int64_t* __restrict__ str_
             bad |= (hi & (neg ? 2 : 1)) || x >= ((int64_t)1 << 31) || x <= -((int64_t)1 << 31);
             u = (uint32_t)x;
         }
-        const uint32_t so = warp_scan_u32(ends && (jl & 1) ? u : 0u, lane);
-        const uint32_t se = warp_scan_u32(ends && !(jl & 1) && jl >= 2 ? u : 0u, lane);
+        const uint32_t so = warp_incl_scan(ends && (jl & 1) ? u : 0u);
+        const uint32_t se = warp_incl_scan(ends && !(jl & 1) && jl >= 2 ? u : 0u);
         if (ends) {
             const uint32_t cnt = jl == 0 ? u : (jl & 1) ? chain_odd + so : chain_even + se;
             bad |= cnt >= 0x80000000u;
@@ -164,9 +134,7 @@ rd_scan_kernel(const int32_t* __restrict__ counts, const int64_t* __restrict__ c
     int64_t carry = 0;
     for (int64_t base = 0; base < nc; base += 32) {
         const int64_t i = base + lane;
-        int64_t incl = i < nc ? (int64_t)(uint32_t)counts[c0 + i] : 0;    // maskApi's counts are unsigned
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int64_t u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
+        const int64_t incl = warp_incl_scan<int64_t>(i < nc ? (uint32_t)counts[c0 + i] : 0u);  // maskApi's counts are unsigned
         if (i < nc) st[i + 1] = carry + incl;
         carry += __shfl_sync(0xffffffffu, incl, 31);
     }
@@ -266,8 +234,7 @@ extern "C" int s2d_rle_from_strings(const char* chars, const int64_t* str_offset
     const unsigned blocks = (unsigned)((N + RP_WARPS - 1) / RP_WARPS);
     rp_count_kernel<<<blocks, RP_WARPS * 32, 0, st>>>(chars, str_offsets, N, work);
     S2D_CHECK_LAUNCH("rp_count_kernel");
-    rp_scan_kernel<<<1, RP_SCAN_THREADS, 0, st>>>(work, N, count_offsets, needed);
-    S2D_CHECK_LAUNCH("rp_scan_kernel");
+    if (const int rc = launch_offsets(work, N, count_offsets, needed, st)) return rc;
     rp_write_kernel<<<blocks, RP_WARPS * 32, 0, st>>>(chars, str_offsets, N, count_offsets, capacity, counts, status);
     S2D_CHECK_LAUNCH("rp_write_kernel");
     return 0;

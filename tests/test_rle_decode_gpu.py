@@ -69,6 +69,18 @@ def test_parse_equals_from_string():
     assert np.array_equal(c2.cpu().numpy()[:o2[-1]], counts[:coff[40]])
 
 
+@pytest.mark.parametrize("n", [1, 31, 1023, 1024, 1025, 2048, 2049, 5000])
+def test_parse_offsets_across_scan_blocks(n):
+    """count_offsets of n strings, n on both sides of the 1024-element steps of the single-CTA offsets scan"""
+    rng = np.random.default_rng(n)
+    lists = [rng.integers(0, 3000, size=rng.integers(0, 40)).tolist() for _ in range(n)]
+    blobs = [coco_rle.to_string(x).encode() for x in lists]
+    counts, coff, status, need, _ = _parse_cabi(blobs)
+    want = np.zeros(n + 1, np.int64)
+    want[1:] = np.cumsum([len(x) for x in lists])
+    assert np.array_equal(coff, want) and need == coff[-1] and (status == 0).all()
+
+
 def test_parse_flags_malformed_without_disturbing_neighbours():
     rng = np.random.default_rng(1)
     good = [rng.integers(0, 3000, size=rng.integers(1, 200)).tolist() for _ in range(64)]

@@ -113,6 +113,31 @@ def test_overflow_reports_need_and_batch_retries():
     assert _check_rows(b, labs, tab) == rows
 
 
+@pytest.mark.parametrize("n", [1, 31, 1023, 1024, 1025, 2048, 2049, 5000])
+def test_rle_strings_offsets_across_scan_blocks(n):
+    """s2d_rle_strings of n run-length lists, n on both sides of the 1024-element steps of the single-CTA offsets scan"""
+    from s2d_b200 import _lib
+    from s2d_b200.keymask_ident.annotations import coco_rle
+    rng = np.random.default_rng(n)
+    lists = [rng.integers(0, 5000, size=rng.integers(1, 40)).tolist() for _ in range(n)]
+    strings = [coco_rle.to_string(x) for x in lists]
+    offs = np.zeros(n + 1, np.int64)
+    offs[1:] = np.cumsum([len(x) for x in lists])
+    want = np.zeros(n + 1, np.int64)
+    want[1:] = np.cumsum([len(s) for s in strings])
+    counts = torch.from_numpy(np.concatenate(lists).astype(np.int32)).to(DEV)
+    d_off = torch.from_numpy(offs).to(DEV)
+    work = torch.empty(n, dtype=torch.int32, device=DEV)
+    chars = torch.empty(int(want[-1]), dtype=torch.uint8, device=DEV)
+    soff = torch.full((n + 1,), -1, dtype=torch.int64, device=DEV)
+    need = torch.full((1,), -1, dtype=torch.int64, device=DEV)
+    _lib.call("s2d_rle_strings", counts.data_ptr(), d_off.data_ptr(), n, int(offs[-1]), work.data_ptr(), int(want[-1]),
+              chars.data_ptr(), soff.data_ptr(), need.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    torch.cuda.synchronize()
+    assert np.array_equal(soff.cpu().numpy(), want) and int(need.item()) == want[-1]
+    assert chars.cpu().numpy().tobytes().decode("ascii") == "".join(strings)
+
+
 def _groups_from_files(files):
     """(cluster, group) -> {frame: largest mask id} from the reference's group_files (tie rule of the batched path)."""
     out = {}

@@ -140,7 +140,7 @@ def main():
         "steps": args.steps, "warmup": args.warmup,
         "parse": {"strings": nstr, "chars": nchars, "counts": ncounts, "device_ms": {"median": med(t_parse), "all": t_parse},
                   "host_from_string_s": t_host, "equal_to_from_string": parse_equal,
-                  "note": "CUDA events around s2d_rle_from_strings (rp_count_kernel, rp_scan_kernel, rp_write_kernel); "
+                  "note": "CUDA events around s2d_rle_from_strings (rp_count_kernel, offsets_kernel, rp_write_kernel); "
                           "host: coco_rle.from_string over the same strings, one pass"},
         "decode_one_video": {"video": v0, "masks": m, "H": H, "W": W, "counts": vn, "ms": {"median": med(t_dec), "all": t_dec},
                           "bytes_written": written, "write_gbs": gbs, "copy_peak_gbs": COPY_PEAK_GBS,

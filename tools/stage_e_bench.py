@@ -129,7 +129,7 @@ def main():
         torch.cuda.synchronize()
     for e in prof.key_averages():
         if e.key.startswith(("void s2d::lr_", "void s2d::rs_", "s2d::lr_", "s2d::rs_")) or "lr_strip" in e.key or "rs_kernel" in e.key \
-                or "lr_scan" in e.key or "lr_diff" in e.key or "lr_frame" in e.key:
+                or "offsets_kernel" in e.key or "lr_diff" in e.key or "lr_frame" in e.key:
             kern[e.key] = {"calls": e.count, "avg_us": (getattr(e, "device_time", None) or e.cuda_time)}
 
     # previous route on 4 videos: materialised keymask planes -> s2d_rle_encode -> host packer
